@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--only]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # the reference's CPU algorithm (oracle port) on the host cores
+    python bench.py --dump-outputs DIR        # also write a seeded sample of every workload's outputs to DIR/<name>.npy
 
 A step = one pass of the hot path over one batch of synthetic images.  The headline workload (`--workload`,
 default restart8 = BASELINE configs[1]) fills the top-level keys of the JSON line:
@@ -19,6 +20,8 @@ reported under "workloads": norestart (configs[2]: 8192 images over the ranks wh
 encode (configs[4]), plus restart8rgb and restart120 (one MCU row per restart interval: the no-cliff check).
 Every workload is checked against the oracle outside its timed region ("parity_checked": images compared bit for bit).
 Images are sharded by batch index (weak scaling: a fixed batch per GPU), no collective on the data path.
+The inputs are seeded, so the same arguments give the same images on every run and `--dump-outputs` files of two builds
+can be compared value for value.
 The synthetic JPEGs are produced by the product's own GPU encoder (byte-identical to the model's encoder,
 tests/test_gpu_encode.py); oracle/ is executed only as the checker and for cpu_baseline / --impl reference.
 """
@@ -50,6 +53,7 @@ WORKLOADS = {
 }
 EXTRAS = ["norestart", "4k444rgb", "encode", "restart8rgb", "restart120"]
 PARITY_IMAGES = 4
+DUMP_VALUES = 1 << 21  # values per workload that --dump-outputs keeps: 8 MB of float32, all six workloads under 64 MB
 
 
 def _synth_one(args):
@@ -240,6 +244,17 @@ def emit(obj):
         os.write(_REAL_STDOUT, data)
 
 
+def dump_outputs(dirname, name, arrays):
+    """DIR/<name>.npy: float32 of shape (images, k), row i holding k values of arrays[i] (what the caller received for image
+    i) at seeded relative positions.  The positions depend only on the array lengths, so two builds with the same outputs
+    write the same file."""
+    k = max(1, DUMP_VALUES // len(arrays))
+    u = np.random.default_rng(0).random((len(arrays), k))
+    rows = [np.asarray(a)[(u[i] * len(a)).astype(np.int64)] for i, a in enumerate(arrays)]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), np.asarray(rows, np.float32))
+
+
 def workload_config(name, batch_n, unique):
     w, h, chroma, quality, ri, out_name, _ = WORKLOADS[name]
     return {"workload": "%s: %d x %dx%d %d q%d %s per GPU -> %s" % (
@@ -263,8 +278,9 @@ class Env:
         self.ctx, self.world, self.barrier, self.max_over_ranks, self.sampler = ctx, world, barrier, max_over_ranks, sampler
 
 
-def run_decode(env, name, frames, batch_n, steps, warmup, e2e_steps, parity=PARITY_IMAGES):
-    """One decode workload: resident (`value`), per-stage roofline, end to end, oracle check of `parity` images."""
+def run_decode(env, name, frames, batch_n, steps, warmup, e2e_steps, parity=PARITY_IMAGES, dump_dir=None):
+    """One decode workload: resident (`value`), per-stage roofline, end to end, oracle check of `parity` images; with
+    `dump_dir`, a sample of the frames the last timed step decoded goes to dump_dir/<name>.npy."""
     import hcjpeg
 
     ctx = env.ctx
@@ -296,14 +312,16 @@ def run_decode(env, name, frames, batch_n, steps, warmup, e2e_steps, parity=PARI
     ms = ctx.timer_stop()
     env.barrier()
     ms_per_step = env.max_over_ranks(ms) / steps
+    outs, st = b.fetch()  # the frames of the last timed step
+    assert all(s == 0 for s in st), [s for s in st if s][:4]
+    if dump_dir:
+        dump_outputs(dump_dir, name, outs)
     # per-stage timing for the roofline of the dominant kernel (separate passes, same stream, CUDA events)
     stages = {}
     for _ in range(steps):
         for k, v in b.decode_stages().items():
             stages[k] = stages.get(k, 0.0) + v / steps
     clocks = env.sampler.snapshot()
-    outs, st = b.fetch()
-    assert all(s == 0 for s in st), [s for s in st if s][:4]
     nblocks = sum(f.nblocks for f in b.infos)
     out_bytes = sum(hcjpeg.out_size(f, mode) for f in b.infos)
     launches = b.kernels() * steps
@@ -396,8 +414,10 @@ def run_decode(env, name, frames, batch_n, steps, warmup, e2e_steps, parity=PARI
     return res, jpgs
 
 
-def run_encode(env, name, frames, batch_n, steps, warmup, parity=PARITY_IMAGES):
-    """Encode workload: frames in pinned host memory -> files in pinned host memory through hcj_encode_batch."""
+def run_encode(env, name, frames, batch_n, steps, warmup, parity=PARITY_IMAGES, dump_dir=None):
+    """Encode workload: frames in pinned host memory -> files in pinned host memory through hcj_encode_batch.  With
+    `dump_dir`, the file lengths of the last timed step go to dump_dir/<name>_lengths.npy and a sample of the files'
+    bytes to dump_dir/<name>.npy."""
     import hcjpeg
 
     ctx = env.ctx
@@ -447,6 +467,9 @@ def run_encode(env, name, frames, batch_n, steps, warmup, parity=PARITY_IMAGES):
     env.barrier()
     dt = env.max_over_ranks(time.perf_counter() - t0) / steps
     assert all(status[i] == 0 for i in range(batch_n))
+    if dump_dir:
+        dump_outputs(dump_dir, name, [np.ctypeslib.as_array(C.cast(op[i], C.POINTER(C.c_uint8)), shape=(lens[i],)) for i in range(batch_n)])
+        np.save(os.path.join(dump_dir, name + "_lengths.npy"), np.array(lens[:batch_n], np.float64))
     # ---- parity: byte-identical files versus the oracle encoder
     import multiprocessing as mp
 
@@ -481,6 +504,7 @@ def main():
     # Libraries print to stdout on their own (NCCL announces its version there at communicator creation): everything
     # but the JSON line goes to stderr.
     global _REAL_STDOUT
+    sys.dont_write_bytecode = True  # the run leaves the tree as it found it (no __pycache__ of the modules imported from it)
     sys.stdout.flush()
     _REAL_STDOUT = os.dup(1)
     os.dup2(2, 1)
@@ -495,7 +519,13 @@ def main():
     ap.add_argument("--unique", type=int, default=64, help="distinct images cycled to fill the batch")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write a seeded sample of what each timed workload computed in its last step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -572,11 +602,12 @@ def main():
               lambda x: shard.max_over_ranks(x, dist_mod, "cuda"), sampler)
 
     e2e_steps = 0 if args.no_e2e else max(1, min(args.steps, 3))
+    dump_dir = args.dump_outputs if rank == 0 else None
     if args.workload != "encode":
-        result, jpgs = run_decode(env, args.workload, frames, batch_n, args.steps, args.warmup, e2e_steps)
+        result, jpgs = run_decode(env, args.workload, frames, batch_n, args.steps, args.warmup, e2e_steps, dump_dir=dump_dir)
         cpu_items, cpu_kind = jpgs, "decode"
     else:
-        result = run_encode(env, args.workload, frames, batch_n, args.steps, args.warmup)
+        result = run_encode(env, args.workload, frames, batch_n, args.steps, args.warmup, dump_dir=dump_dir)
         cpu_items, cpu_kind = frames, "encode"
 
     workloads = {}
@@ -586,9 +617,9 @@ def main():
         fr = extra_frames[(ew, eh, ec)]
         steps = max(1, min(args.steps, 10))
         if name == "encode":
-            r = run_encode(env, name, fr, bn, steps, 3)
+            r = run_encode(env, name, fr, bn, steps, 3, dump_dir=dump_dir)
         else:
-            r, _ = run_decode(env, name, fr, bn, steps, 3, 0 if args.no_e2e else min(2, steps))
+            r, _ = run_decode(env, name, fr, bn, steps, 3, 0 if args.no_e2e else min(2, steps), dump_dir=dump_dir)
         workloads[name] = r
 
     sampler.stop()
