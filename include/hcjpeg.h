@@ -234,6 +234,34 @@ int hcj_encode_batch(hcj_ctx *ctx, const uint8_t *const *yuv, int n, int width, 
 int hcj_encode_batch_multi(hcj_ctx *const *ctx, int nctx, const uint8_t *const *yuv, int n, int width, int height, int chroma,
                            int quality, int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
                            int *status);
+/* The same for RGB24 frames (extension; the model's encoder takes planar frames only): rgb[i] is width*height*3 bytes,
+ * R, G, B interleaved, rows top to bottom, no padding - the layout HCJ_OUT_RGB24 decodes to.  On the device, every frame
+ * is taken to the planar frame of `chroma` that hcj_encode_batch would be given, in two steps:
+ *   1. JFIF full-range forward conversion, libjpeg's jccolor.c in 16-bit fixed point with arithmetic shifts (every
+ *      result lies in [0, 255]; each channel is within 1 of OpenCV's COLOR_RGB2YCrCb and Pillow's "YCbCr"):
+ *        Y  = ( 19595 R + 38470 G +  7471 B + 32768)               >> 16
+ *        Cb = (-11059 R - 21709 G + 32768 B + (128 << 16) + 32767) >> 16
+ *        Cr = ( 32768 R - 27439 G -  5329 B + (128 << 16) + 32767) >> 16
+ *   2. chroma 420 / 422: Planar_444.convert_to_420 / convert_to_422 (tools/src/planar_444.ml:18-23,68-80) of the
+ *      rounded 4:4:4 Cb / Cr planes: planes of floor(width/2) x floor(height/2) (or x height), the average of each 2x2
+ *      (2x1) group with rounding, an odd last column or row dropped.  444 keeps the planes, 400 keeps Y only.
+ * That frame is then encoded exactly as hcj_encode_batch encodes it: the files are byte-identical, statuses (for
+ * example HCJ_ERR_PLANE_BOUNDS), out_len, HCJ_ERR_BUFFER_TOO_SMALL, hcj_encode_bound and hcj_encode_last_device_ms
+ * (which includes the conversion) behave the same.  Without flags the frames are in host memory and go up chunk by
+ * chunk like planar frames (3 bytes a pixel instead of 1.5 for 4:2:0).  flags: HCJ_ENC_SRC_DEVICE, or 0; other bits
+ * are HCJ_ERR_INVALID_ARG. */
+#define HCJ_ENC_SRC_DEVICE 1u /* rgb[i] are device pointers on the context's device */
+/* With HCJ_ENC_SRC_DEVICE nothing is uploaded: the conversion reads the caller's buffers, on the context's stream (the
+ * one passed to hcj_ctx_create), so work the caller enqueued on that stream before the call is ordered before the
+ * reads; work on other streams must be synchronised by the caller.  Every pointer is checked before any work is
+ * enqueued: one that is not device (or managed) memory of the context's device makes the call return
+ * HCJ_ERR_INVALID_ARG with nothing written.  As everywhere, nothing reads caller memory after the call returns. */
+int hcj_encode_rgb_batch(hcj_ctx *ctx, const uint8_t *const *rgb, int n, int width, int height, int chroma, int quality,
+                         int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity,
+                         size_t *out_len, int *status);
+/* The conversion alone (steps 1-2), one frame, host buffers: the planar frame hcj_encode_rgb_batch encodes
+ * (width*height bytes of Y, then Cb and Cr; Y only for 400).  HCJ_ERR_BUFFER_TOO_SMALL if dst_capacity is less. */
+int hcj_rgb_to_yuv(hcj_ctx *ctx, const uint8_t *rgb, int width, int height, int chroma, uint8_t *dst, size_t dst_capacity);
 size_t hcj_encode_bound(int width, int height, int chroma); /* worst-case bytes of one encoded frame */
 int hcj_encode_count_kernels(void); /* kernels one hcj_encode_batch launches */
 /* Encoder.write_headers (encoder.ml:371-418).  Host only. */

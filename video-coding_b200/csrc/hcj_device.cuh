@@ -1128,4 +1128,60 @@ HCJ_HD int32_t packed_coef(const uint32_t *qw, int k) {
   return (k & 1) ? (int32_t)w >> 16 : (int32_t)(int16_t)(w & 0xffffu);
 }
 
+
+// ------------------------------------------------------------------------------------------------
+// Stated forward colour conversion (DESIGN.md 5; not in the reference): JFIF full range, libjpeg's jccolor.c in 16-bit
+// fixed point.  Returns the sums before the shift: sample = t >> 16, and every t lies in [0, 2^24), so the sample is
+// byte 2 of t and no clamp is needed (all 2^24 triples checked, tests/test_encode_rgb.py).
+// ------------------------------------------------------------------------------------------------
+HCJ_HD void rgb_to_ycc_fixed(int r, int g, int b, int &ty, int &tcb, int &tcr) {
+  ty = 19595 * r + 38470 * g + 7471 * b + 32768;
+  tcb = -11059 * r - 21709 * g + 32768 * b + ((128 << 16) + 32767);
+  tcr = 32768 * r - 27439 * g - 5329 * b + ((128 << 16) + 32767);
+}
+
+#if defined(__CUDACC__)
+// NW words to `nbytes` bytes at any address: 16-byte stores when the address allows and all bytes are wanted,
+// 4-byte stores when it is word aligned, bytes otherwise (and for the tail).
+template <int NW>
+__device__ __forceinline__ void store_any(uint8_t *dst, const uint32_t (&w)[NW], int nbytes) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(dst);
+  if (NW % 4 == 0 && (a & 15u) == 0 && nbytes == NW * 4) {
+#pragma unroll
+    for (int k = 0; k < NW / 4; k++) reinterpret_cast<uint4 *>(dst)[k] = make_uint4(w[4 * k], w[4 * k + 1], w[4 * k + 2], w[4 * k + 3]);
+  } else if ((a & 3u) == 0) {
+#pragma unroll
+    for (int k = 0; k < NW; k++) {
+      if (4 * k + 4 <= nbytes) {
+        reinterpret_cast<uint32_t *>(dst)[k] = w[k];
+      } else {
+#pragma unroll
+        for (int i = 0; i < 4; i++)
+          if (4 * k + i < nbytes) dst[4 * k + i] = (uint8_t)(w[k] >> (8 * i));
+      }
+    }
+  } else {
+    // not word aligned: up to three head bytes, then the words of the byte sequence shifted by the head (funnel
+    // shifts over neighbouring words), then up to three tail bytes - instead of a byte store per byte
+    const int head = (4 - (int)(a & 3u)) & 3, sh = 8 * head;
+#pragma unroll
+    for (int i = 0; i < 3; i++)
+      if (i < head && i < nbytes) dst[i] = (uint8_t)(w[0] >> (8 * i));
+    const int nw = nbytes > head ? (nbytes - head) >> 2 : 0;
+    uint32_t *d32 = reinterpret_cast<uint32_t *>(dst + head);
+    uint32_t tail = 0;
+#pragma unroll
+    for (int k = 0; k < NW; k++) {
+      const uint32_t v = __funnelshift_r(w[k], k + 1 < NW ? w[k + 1] : 0u, sh);  // bytes head + 4k .. head + 4k + 3
+      if (k < nw) d32[k] = v;
+      if (k == nw) tail = v;
+    }
+    const int done = head + 4 * nw;
+#pragma unroll
+    for (int i = 0; i < 3; i++)
+      if (done + i < nbytes) dst[done + i] = (uint8_t)(tail >> (8 * i));
+  }
+}
+#endif
+
 }  // namespace hcjdev

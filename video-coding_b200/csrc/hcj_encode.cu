@@ -14,6 +14,8 @@
 //   k_seg_count    E9        per unit (segment, or 1 KiB of a lone segment): stuffed byte count
 //   k_seg_scan     per frame: prefix sum of unit sizes -> output offsets; copies the header
 //   k_stuff        E9,E10    per unit: byte copy with FF -> FF 00, RSTn between segments, EOI
+//   k_rgb_to_ycc   K10       RGB24 input only (hcj_encode_rgb_batch): stated RGB -> YCbCr + Planar_444.convert_to_420 / _422
+//                            into the planar frame buffer k_fdct_quant reads, from uploaded frames or the caller's device buffers
 //
 // Results are byte-identical to the model's Writer.get_buffer (tests/test_gpu_encode.py).
 #include <cuda_runtime.h>
@@ -522,6 +524,179 @@ __global__ void __launch_bounds__(128) k_stuff(EncodeBatchDev e) {
   }
 }
 
+// ---- K10 -----------------------------------------------------------------------------------------
+// RGB24 frames -> the planar frames k_fdct_quant reads (Frame.input layout: Y of w x h, then Cb and Cr of the chroma
+// plane's size; Y only for 400).  The stated forward conversion (rgb_to_ycc_fixed, DESIGN.md 5), then
+// Planar_444.convert_to_420 / _422 (planar_444.ml:18-23,68-80) over the ROUNDED 4:4:4 chroma samples: an odd last
+// column or row of 4:4:4 chroma is dropped.  A bandwidth kernel like k_rgb_sub_pairs in the other direction: one
+// thread per group of 16 pixels (of two rows for 4:2:0, which share their chroma samples), every load issued before any
+// arithmetic, 16-byte loads (a row that is not 16-byte aligned is realigned from the aligned chunks around it with
+// funnel shifts), alignment-adaptive stores.  Frames come from a device-side pointer table, so uploaded frames and the
+// caller's device buffers take the same code.
+struct RgbToYcc {
+  const uint8_t *const *rgb;  // [frames] w * h * 3 bytes each
+  uint8_t *dst;               // [frames][frame_bytes]
+  uint64_t frame_bytes, off_cb, off_cr;
+  int w, h, cw;               // cw: width of the chroma planes
+  uint32_t groups, sets;      // 16-pixel groups per row; row sets (pairs of rows for 4:2:0) per frame
+};
+
+// The aligned 16-byte chunks that hold the 48 bytes at p: three when p is 16-byte aligned, four otherwise.  Each chunk
+// holds at least one of the 48 bytes, so nothing is read outside the 16-byte granules of the row.
+__device__ __forceinline__ void load48_raw(const uint8_t *p, uint32_t (&u)[16]) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(p);
+  const uint4 *q = reinterpret_cast<const uint4 *>(a & ~(uintptr_t)15);
+#pragma unroll
+  for (int k = 0; k < 3; k++) {
+    const uint4 v = __ldg(q + k);
+    u[4 * k] = v.x, u[4 * k + 1] = v.y, u[4 * k + 2] = v.z, u[4 * k + 3] = v.w;
+  }
+  uint4 v = make_uint4(0u, 0u, 0u, 0u);
+  if (a & 15u) v = __ldg(q + 3);
+  u[12] = v.x, u[13] = v.y, u[14] = v.z, u[15] = v.w;
+}
+// The 48 bytes at p as 12 words, from the chunks load48_raw fetched: a word shift by selects, then a byte shift.
+__device__ __forceinline__ void align48(const uint8_t *p, const uint32_t (&u)[16], uint32_t (&w)[12]) {
+  const uint32_t a = (uint32_t)reinterpret_cast<uintptr_t>(p) & 15u;
+  if (a == 0u) {
+#pragma unroll
+    for (int k = 0; k < 12; k++) w[k] = u[k];
+    return;
+  }
+  const uint32_t q = a >> 2, sh = 8u * (a & 3u);
+  uint32_t v[13];
+#pragma unroll
+  for (int k = 0; k < 13; k++) v[k] = q == 0u ? u[k] : q == 1u ? u[k + 1] : q == 2u ? u[k + 2] : u[k + 3];
+#pragma unroll
+  for (int k = 0; k < 12; k++) w[k] = __funnelshift_r(v[k], v[k + 1], sh);
+}
+__device__ __forceinline__ int rgb_byte(const uint32_t (&w)[12], int j) { return (int)__byte_perm(w[j >> 2], 0u, 0x4440u | (j & 3)); }
+// byte 2 (the sample, see rgb_to_ycc_fixed) of four sums -> one word
+__device__ __forceinline__ uint32_t pack_b2(int t0, int t1, int t2, int t3) {
+  return __byte_perm(__byte_perm(t0, t1, 0x0062u), __byte_perm(t2, t3, 0x0062u), 0x5410u);
+}
+__device__ __forceinline__ uint32_t pack_b0(int c0, int c1, int c2, int c3) {
+  return __byte_perm(__byte_perm(c0, c1, 0x0040u), __byte_perm(c2, c3, 0x0040u), 0x5410u);
+}
+
+// The short last group of a row (n < 16 pixels, which is where an odd last column lies), and the lone last row of a
+// 4:2:0 frame of odd height: byte by byte.
+template <int CHROMA>
+__device__ __forceinline__ void rgb_to_ycc_tail(const uint8_t *src, int w, int n, bool two, uint8_t *dy, uint8_t *dcb, uint8_t *dcr) {
+  const int rows = two ? 2 : 1;
+  for (int r = 0; r < rows; r++)
+    for (int i = 0; i < n; i++) {
+      const uint8_t *p = src + ((size_t)r * w + i) * 3;
+      int ty, tcb, tcr;
+      rgb_to_ycc_fixed(p[0], p[1], p[2], ty, tcb, tcr);
+      dy[(size_t)r * w + i] = (uint8_t)(ty >> 16);
+      if (CHROMA == 444) dcb[i] = (uint8_t)(tcb >> 16), dcr[i] = (uint8_t)(tcr >> 16);
+    }
+  if constexpr (CHROMA == 420 || CHROMA == 422) {
+    if (CHROMA == 420 && !two) return;
+    for (int j = 0; j < n / 2; j++) {
+      int sb = 0, sr = 0;
+      for (int r = 0; r < rows; r++)
+        for (int i = 2 * j; i < 2 * j + 2; i++) {
+          const uint8_t *p = src + ((size_t)r * w + i) * 3;
+          int ty, tcb, tcr;
+          rgb_to_ycc_fixed(p[0], p[1], p[2], ty, tcb, tcr);
+          sb += tcb >> 16, sr += tcr >> 16;
+        }
+      dcb[j] = (uint8_t)(CHROMA == 420 ? (sb + 2) >> 2 : (sb + 1) >> 1);  // avg4 / avg2 (planar_444.ml:4-16)
+      dcr[j] = (uint8_t)(CHROMA == 420 ? (sr + 2) >> 2 : (sr + 1) >> 1);
+    }
+  }
+}
+
+template <int CHROMA>
+__global__ void __launch_bounds__(128, 8) k_rgb_to_ycc(RgbToYcc a) {
+  constexpr int ROWS = CHROMA == 420 ? 2 : 1;
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x, set = t / a.groups, g = t - set * a.groups;
+  if (set >= a.sets) return;
+  const int x0 = (int)g * 16, y0 = (int)set * ROWS, n = min(16, a.w - x0);
+  const bool two = ROWS == 2 && y0 + 1 < a.h;
+  const uint8_t *src = a.rgb[blockIdx.y] + ((size_t)y0 * a.w + x0) * 3;
+  uint8_t *frame = a.dst + (uint64_t)blockIdx.y * a.frame_bytes;
+  uint8_t *dy = frame + (size_t)y0 * a.w + x0;
+  uint8_t *dcb = frame + a.off_cb + (size_t)set * a.cw + (CHROMA == 444 ? x0 : x0 / 2), *dcr = dcb + (a.off_cr - a.off_cb);
+  if (n < 16 || (ROWS == 2 && !two)) {
+    rgb_to_ycc_tail<CHROMA>(src, a.w, n, two, dy, dcb, dcr);
+    return;
+  }
+  uint32_t u0[16], u1[16], w0[12], w1[12];
+  load48_raw(src, u0);
+  if (ROWS == 2) load48_raw(src + (size_t)a.w * 3, u1);
+  align48(src, u0, w0);
+  if (ROWS == 2) align48(src + (size_t)a.w * 3, u1, w1);
+  uint32_t oy0[4], oy1[4], ocb[4], ocr[4];
+  int cb[8], cr[8];
+#pragma unroll
+  for (int q = 0; q < 4; q++) {  // pixels 4q .. 4q + 3
+    int ty[4], tb[4], tr[4], uy[4], ub[4], ur[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      const int j = 3 * (4 * q + i);
+      rgb_to_ycc_fixed(rgb_byte(w0, j), rgb_byte(w0, j + 1), rgb_byte(w0, j + 2), ty[i], tb[i], tr[i]);
+      if (ROWS == 2) rgb_to_ycc_fixed(rgb_byte(w1, j), rgb_byte(w1, j + 1), rgb_byte(w1, j + 2), uy[i], ub[i], ur[i]);
+    }
+    oy0[q] = pack_b2(ty[0], ty[1], ty[2], ty[3]);
+    if (ROWS == 2) oy1[q] = pack_b2(uy[0], uy[1], uy[2], uy[3]);
+    if (CHROMA == 444) {
+      ocb[q] = pack_b2(tb[0], tb[1], tb[2], tb[3]);
+      ocr[q] = pack_b2(tr[0], tr[1], tr[2], tr[3]);
+    }
+#pragma unroll
+    for (int k = 0; k < 2; k++) {  // avg4 / avg2 (planar_444.ml:4-16) of the rounded samples
+      if (CHROMA == 420) {
+        cb[2 * q + k] = ((tb[2 * k] >> 16) + (tb[2 * k + 1] >> 16) + (ub[2 * k] >> 16) + (ub[2 * k + 1] >> 16) + 2) >> 2;
+        cr[2 * q + k] = ((tr[2 * k] >> 16) + (tr[2 * k + 1] >> 16) + (ur[2 * k] >> 16) + (ur[2 * k + 1] >> 16) + 2) >> 2;
+      } else if (CHROMA == 422) {
+        cb[2 * q + k] = ((tb[2 * k] >> 16) + (tb[2 * k + 1] >> 16) + 1) >> 1;
+        cr[2 * q + k] = ((tr[2 * k] >> 16) + (tr[2 * k + 1] >> 16) + 1) >> 1;
+      }
+    }
+  }
+  store_any<4>(dy, oy0, 16);
+  if (ROWS == 2) store_any<4>(dy + a.w, oy1, 16);
+  if (CHROMA == 444) {
+    store_any<4>(dcb, ocb, 16);
+    store_any<4>(dcr, ocr, 16);
+  } else if (CHROMA != 400) {
+    const uint32_t sb[2] = {pack_b0(cb[0], cb[1], cb[2], cb[3]), pack_b0(cb[4], cb[5], cb[6], cb[7])};
+    const uint32_t sr[2] = {pack_b0(cr[0], cr[1], cr[2], cr[3]), pack_b0(cr[4], cr[5], cr[6], cr[7])};
+    store_any<2>(dcb, sb, 8);
+    store_any<2>(dcr, sr, 8);
+  }
+}
+
+uint64_t rgb_frame_planar_bytes(int w, int h, int chroma) {  // Frame.create (frame.ml:32-40); one plane for 400
+  return chroma == 400 ? (uint64_t)w * h : yuv_frame_bytes(w, h, chroma);
+}
+
+void launch_rgb_to_ycc(const uint8_t *const *rgb, int frames, int w, int h, int chroma, uint8_t *dst, cudaStream_t s) {
+  if (frames <= 0 || w <= 0 || h <= 0) return;
+  RgbToYcc a;
+  a.rgb = rgb;
+  a.dst = dst;
+  a.w = w;
+  a.h = h;
+  a.cw = chroma == 444 ? w : w / 2;
+  const int ch = chroma == 420 ? h / 2 : h;
+  a.frame_bytes = rgb_frame_planar_bytes(w, h, chroma);
+  a.off_cb = (uint64_t)w * h;
+  a.off_cr = a.off_cb + (uint64_t)a.cw * ch;
+  a.groups = (uint32_t)((w + 15) / 16);
+  a.sets = (uint32_t)(chroma == 420 ? (h + 1) / 2 : h);
+  const dim3 grid((unsigned)(((uint64_t)a.groups * a.sets + 127) / 128), (unsigned)frames);
+  switch (chroma) {
+    case 420: k_rgb_to_ycc<420><<<grid, 128, 0, s>>>(a); break;
+    case 422: k_rgb_to_ycc<422><<<grid, 128, 0, s>>>(a); break;
+    case 444: k_rgb_to_ycc<444><<<grid, 128, 0, s>>>(a); break;
+    default: k_rgb_to_ycc<400><<<grid, 128, 0, s>>>(a); break;
+  }
+}
+
 void launch_encode(const EncodeBatchDev &e, cudaStream_t s) {
   if (e.n == 0) return;
   dim3 gb((e.nblocks + 127) / 128, e.n);
@@ -789,14 +964,24 @@ int hcj_write_headers(int width, int height, int chroma, int quality, int restar
   return HCJ_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+// Where the frames of a chunk come from: the only stage in which the encode entry points differ.
+enum class EncodeSource {
+  YUV_HOST,    // planar frames in host memory: uploaded into the chunk's slot, which k_fdct_quant reads
+  RGB_HOST,    // RGB24 frames in host memory: uploaded into the chunk's slot, converted by k_rgb_to_ycc into e.src
+  RGB_DEVICE,  // RGB24 frames in device memory: converted by k_rgb_to_ycc straight from the caller's buffers into e.src
+};
+
 // Frames go through the device in chunks: while the kernels of chunk k run, the frames of chunk k + 1 go up on a second
 // stream and the files of chunk k - 1 come down on a third (the call used to be H2D, then kernels, then D2H: 41.8 ms per
 // 512 x 1080p frames, of which 29 ms is the 1.6 GB of frames on the PCIe link).  The host waits twice per chunk for the
 // kernel stream only - for the bit totals that size the byte buffers, and for the file lengths - which the copies on
-// the other two streams do not notice.  Source frames and finished files are double-buffered on the device.
-int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
-                     int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len, int *status) {
-  if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!yuv || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
+// the other two streams do not notice.  Uploaded frames and finished files are double-buffered on the device.
+int encode_frames(hcj_ctx *c, EncodeSource kind, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
+                  int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len, int *status) {
   CU_TRY(cudaSetDevice(c->device));
   int chunk = 64;
   if (const char *ev = getenv("HCJ_ENC_CHUNK")) chunk = std::max(1, atoi(ev));
@@ -812,15 +997,36 @@ int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, in
   cudaError_t err = cudaSuccess;
   c->enc_timed = false;
   c->enc_ms = 0.f;
-  // second slot of source frames; slots of finished files grow on demand
-  uint8_t *src_slot[2] = {const_cast<uint8_t *>(e.src), nullptr};
+  // upload slots: planar frames go straight into e.src and a second slot, RGB frames into two slots of their own in
+  // front of the conversion (whose planar output e.src only the kernel stream touches); slots of finished files grow on
+  // demand
+  const bool rgb = kind != EncodeSource::YUV_HOST;
+  const uint64_t slot_frame = kind == EncodeSource::YUV_HOST ? e.frame_bytes : 3ull * width * height;
+  uint8_t *src_slot[2] = {kind == EncodeSource::YUV_HOST ? const_cast<uint8_t *>(e.src) : nullptr, nullptr};
   uint8_t *out_slot[2] = {nullptr, nullptr};
   uint64_t out_cap[2] = {0, 0}, raw_cap = 0, segb_cap = 0;
-  if (nchunks > 1) {
-    st = c->alloc((void **)&src_slot[1], e.frame_bytes * (uint64_t)ch + 16);
-    if (st == HCJ_OK) S.owned.push_back(src_slot[1]);
-  } else {
-    src_slot[1] = src_slot[0];
+  auto alloc_owned = [&](void **ptr, size_t bytes) {
+    if (st != HCJ_OK) return;
+    st = c->alloc(ptr, bytes);
+    if (st == HCJ_OK) S.owned.push_back(*ptr);
+  };
+  if (kind == EncodeSource::RGB_HOST) alloc_owned((void **)&src_slot[0], slot_frame * (uint64_t)ch + 16);
+  if (kind != EncodeSource::RGB_DEVICE) {
+    if (nchunks > 1) alloc_owned((void **)&src_slot[1], slot_frame * (uint64_t)ch + 16);
+    else src_slot[1] = src_slot[0];
+  }
+  // k_rgb_to_ycc's frame table: the frames of both slots, or every caller frame (chunk k reads entries k * ch ..)
+  const uint8_t **d_frames = nullptr;
+  std::vector<const uint8_t *> frames;
+  if (rgb && st == HCJ_OK) {
+    if (kind == EncodeSource::RGB_HOST)
+      for (int k = 0; k < 2; k++)
+        for (int i = 0; i < ch; i++) frames.push_back(src_slot[k] + (uint64_t)i * slot_frame);
+    else
+      frames.assign(yuv, yuv + n);
+    alloc_owned((void **)&d_frames, frames.size() * sizeof(frames[0]));
+    if (st == HCJ_OK && cudaMemcpyAsync(d_frames, frames.data(), frames.size() * sizeof(frames[0]), cudaMemcpyHostToDevice, c->stream) != cudaSuccess)
+      st = HCJ_ERR_CUDA - (int)cudaGetLastError();
   }
   std::vector<cudaEvent_t> ev_up(nchunks), ev_src_free(nchunks), ev_done(nchunks), ev_down(nchunks), ev_t(4 * (size_t)nchunks);
   for (auto *v : {&ev_up, &ev_src_free, &ev_done, &ev_down})
@@ -833,10 +1039,10 @@ int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, in
   auto upload = [&](int k) {  // frames of chunk k -> their slot, behind the kernels that last read it
     const int lo = k * ch, hi = std::min(n, lo + ch);
     if (k >= 2 && err == cudaSuccess) err = cudaStreamWaitEvent(us, ev_src_free[k - 2], 0);
-    for (int i = lo; i < hi && err == cudaSuccess;) {  // frames that lie back to back in host memory go up as one copy
+    for (int i = lo; i < hi && err == cudaSuccess && kind != EncodeSource::RGB_DEVICE;) {  // frames that lie back to back in host memory go up as one copy
       int j = i + 1;
-      while (j < hi && yuv[j] == yuv[j - 1] + e.frame_bytes) j++;
-      err = cudaMemcpyAsync(src_slot[k & 1] + (uint64_t)(i - lo) * e.frame_bytes, yuv[i], e.frame_bytes * (uint64_t)(j - i), cudaMemcpyHostToDevice, us);
+      while (j < hi && yuv[j] == yuv[j - 1] + slot_frame) j++;
+      err = cudaMemcpyAsync(src_slot[k & 1] + (uint64_t)(i - lo) * slot_frame, yuv[i], slot_frame * (uint64_t)(j - i), cudaMemcpyHostToDevice, us);
       i = j;
     }
     if (err == cudaSuccess) err = cudaEventRecord(ev_up[k], us);
@@ -846,12 +1052,15 @@ int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, in
     const int lo = k * ch, hi = std::min(n, lo + ch), m = hi - lo;
     if (k + 1 < nchunks) upload(k + 1);
     e.n = m;
-    e.src = src_slot[k & 1];
+    if (!rgb) e.src = src_slot[k & 1];
     // phase 1: coefficients and the bit length of every block; the totals size the byte buffers
     if (err == cudaSuccess) err = cudaStreamWaitEvent(s, ev_up[k], 0);
     if (err == cudaSuccess) err = cudaMemsetAsync(S.d_status, 0, 4 * (size_t)m, s);
     if (err == cudaSuccess) err = cudaMemsetAsync(e.long_blocks, 0, 4, s);
     cudaEventRecord(ev_t[4 * k + 0], s);
+    if (rgb)
+      hcjk::launch_rgb_to_ycc(d_frames + (kind == EncodeSource::RGB_HOST ? (k & 1) * ch : lo), m, width, height, chroma,
+                              const_cast<uint8_t *>(e.src), s);
     hcjk::launch_encode(e, s);
     hcjk::launch_bit_lengths(e, S.d_status, e.out_len, s);
     cudaEventRecord(ev_t[4 * k + 1], s);
@@ -919,6 +1128,65 @@ int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, in
   teardown_encode(c, &S);
   if (st != HCJ_OK) return st;
   return err == cudaSuccess ? HCJ_OK : HCJ_ERR_CUDA - (int)err;
+}
+
+}  // namespace
+
+extern "C" {
+
+int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
+                     int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len, int *status) {
+  if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!yuv || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
+  return encode_frames(c, EncodeSource::YUV_HOST, yuv, n, width, height, chroma, quality, restart_interval, out, out_capacity,
+                       out_len, status);
+}
+
+int hcj_encode_rgb_batch(hcj_ctx *c, const uint8_t *const *rgb, int n, int width, int height, int chroma, int quality,
+                         int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
+                         int *status) {
+  if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!rgb || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
+  if (flags & ~HCJ_ENC_SRC_DEVICE) return HCJ_ERR_INVALID_ARG;
+  if (flags & HCJ_ENC_SRC_DEVICE) {  // every frame must be device (or managed) memory of the context's device
+    for (int i = 0; i < n; i++) {
+      cudaPointerAttributes at;
+      if (!rgb[i] || cudaPointerGetAttributes(&at, rgb[i]) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return HCJ_ERR_INVALID_ARG;
+      }
+      if ((at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) || at.device != c->device) return HCJ_ERR_INVALID_ARG;
+    }
+  }
+  return encode_frames(c, (flags & HCJ_ENC_SRC_DEVICE) ? EncodeSource::RGB_DEVICE : EncodeSource::RGB_HOST, rgb, n, width, height,
+                       chroma, quality, restart_interval, out, out_capacity, out_len, status);
+}
+
+int hcj_rgb_to_yuv(hcj_ctx *c, const uint8_t *rgb, int width, int height, int chroma, uint8_t *dst, size_t dst_capacity) {
+  if (!c || !rgb || !dst || width < 1 || height < 1 || (chroma != 420 && chroma != 422 && chroma != 444 && chroma != 400))
+    return HCJ_ERR_INVALID_ARG;
+  const uint64_t nin = 3ull * width * height, nout = hcjk::rgb_frame_planar_bytes(width, height, chroma);
+  if (dst_capacity < nout) return HCJ_ERR_BUFFER_TOO_SMALL;
+  CU_TRY(cudaSetDevice(c->device));
+  void *d_in = nullptr, *d_out = nullptr, *d_tab = nullptr;
+  int st = c->alloc(&d_in, nin + 16);
+  if (st == HCJ_OK) st = c->alloc(&d_out, nout + 16);
+  if (st == HCJ_OK) st = c->alloc(&d_tab, sizeof(void *));
+  cudaError_t e = cudaSuccess;
+  if (st == HCJ_OK) {
+    e = cudaMemcpyAsync(d_in, rgb, nin, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_tab, &d_in, sizeof(void *), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) {
+      hcjk::launch_rgb_to_ycc(static_cast<const uint8_t *const *>(d_tab), 1, width, height, chroma, static_cast<uint8_t *>(d_out), c->stream);
+      e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dst, d_out, nout, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  }
+  cudaStreamSynchronize(c->stream);  // nothing in flight may lose its memory
+  c->release(d_in);
+  c->release(d_out);
+  c->release(d_tab);
+  if (st != HCJ_OK) return st;
+  return e == cudaSuccess ? HCJ_OK : HCJ_ERR_CUDA - (int)e;
 }
 
 // The encoder mirror of hcj_decode_batch_multi: context k encodes frames hcj_shard_range(n, k, nctx) on its own host thread.

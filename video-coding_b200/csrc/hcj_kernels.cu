@@ -1738,47 +1738,6 @@ __device__ __forceinline__ void idct_fetch_record(const DecodeBatchDev &b, IdctT
   asm volatile("cp.async.commit_group;\n" ::: "memory");  // one group per call, empty past the end
 }
 
-// NW words to `nbytes` bytes at any address: 16-byte stores when the address allows and all bytes are wanted,
-// 4-byte stores when it is word aligned, bytes otherwise (and for the tail).
-template <int NW>
-__device__ __forceinline__ void store_any(uint8_t *dst, const uint32_t (&w)[NW], int nbytes) {
-  const uintptr_t a = reinterpret_cast<uintptr_t>(dst);
-  if (NW % 4 == 0 && (a & 15u) == 0 && nbytes == NW * 4) {
-#pragma unroll
-    for (int k = 0; k < NW / 4; k++) reinterpret_cast<uint4 *>(dst)[k] = make_uint4(w[4 * k], w[4 * k + 1], w[4 * k + 2], w[4 * k + 3]);
-  } else if ((a & 3u) == 0) {
-#pragma unroll
-    for (int k = 0; k < NW; k++) {
-      if (4 * k + 4 <= nbytes) {
-        reinterpret_cast<uint32_t *>(dst)[k] = w[k];
-      } else {
-#pragma unroll
-        for (int i = 0; i < 4; i++)
-          if (4 * k + i < nbytes) dst[4 * k + i] = (uint8_t)(w[k] >> (8 * i));
-      }
-    }
-  } else {
-    // not word aligned: up to three head bytes, then the words of the byte sequence shifted by the head (funnel
-    // shifts over neighbouring words), then up to three tail bytes - instead of a byte store per byte
-    const int head = (4 - (int)(a & 3u)) & 3, sh = 8 * head;
-#pragma unroll
-    for (int i = 0; i < 3; i++)
-      if (i < head && i < nbytes) dst[i] = (uint8_t)(w[0] >> (8 * i));
-    const int nw = nbytes > head ? (nbytes - head) >> 2 : 0;
-    uint32_t *d32 = reinterpret_cast<uint32_t *>(dst + head);
-    uint32_t tail = 0;
-#pragma unroll
-    for (int k = 0; k < NW; k++) {
-      const uint32_t v = __funnelshift_r(w[k], k + 1 < NW ? w[k + 1] : 0u, sh);  // bytes head + 4k .. head + 4k + 3
-      if (k < nw) d32[k] = v;
-      if (k == nw) tail = v;
-    }
-    const int done = head + 4 * nw;
-#pragma unroll
-    for (int i = 0; i < 3; i++)
-      if (done + i < nbytes) dst[done + i] = (uint8_t)(tail >> (8 * i));
-  }
-}
 // ------------------------------------------------------------------------------------------------
 // J4: dequantise + IDCT + colour in ONE kernel for RGB24 output of 4:4:4 images (north_star: "dequantisation, 8x8
 // IDCT, upsampling and YCbCr->RGB as one fused kernel"; for 4:4:4 Planar_444 is the identity).  The three blocks of an

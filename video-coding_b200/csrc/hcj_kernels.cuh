@@ -153,5 +153,8 @@ struct EncodeBatchDev {
 void launch_encode(const EncodeBatchDev &e, cudaStream_t s);
 void launch_encode_block_log(const EncodeBatchDev &e, uint32_t first, uint32_t count, void *out /* hcj_encoder_block[count] */, cudaStream_t s);
 int encode_kernel_count();
+// K10: RGB24 frames (device pointer table rgb[frames]) -> planar frames of `chroma` (420 / 422 / 444 / 400), back to back in dst
+void launch_rgb_to_ycc(const uint8_t *const *rgb, int frames, int w, int h, int chroma, uint8_t *dst, cudaStream_t s);
+uint64_t rgb_frame_planar_bytes(int w, int h, int chroma);
 
 }  // namespace hcjk

@@ -22,6 +22,7 @@ OUT_YUV, OUT_PLANES, OUT_RGB24, OUT_YUV444 = 0, 1, 2, 3
 FLAG_RESTART_EXT = 1
 FLAG_T81_TABLES = 2
 FLAG_DEFAULT = FLAG_RESTART_EXT
+ENC_SRC_DEVICE = 1  # hcj_encode_rgb_batch: the frames are device pointers on the context's device
 
 MAX_COMPONENTS = 4
 MAX_TABLE_SEGMENTS = 64
@@ -173,6 +174,8 @@ _SIGS = {
     "hcj_batch_fetch_entropy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, _P(C.c_size_t)]),
     "hcj_idct_blocks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "hcj_encode_batch": (C.c_int, [C.c_void_p, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
+    "hcj_encode_rgb_batch": (C.c_int, [C.c_void_p, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
+    "hcj_rgb_to_yuv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
     "hcj_encode_bound": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "hcj_encode_count_kernels": (C.c_int, []),
     "hcj_write_headers": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, _P(C.c_size_t)]),
@@ -293,6 +296,39 @@ def _ptr_array(bufs):
             arr[i] = C.addressof(cb)
             keep.append(cb)
     return arr, keep
+
+
+def _rgb_frames(frames, width, height, allow_device=True):
+    """Checks RGB24 frames before the library sees them: ([uint8 array, or device address as int], flags).  Host frames:
+    bytes of width*height*3, or C-contiguous uint8 arrays of shape (height, width, 3); device frames: objects with
+    __cuda_array_interface__ of that shape, dtype and (C-contiguous) layout.  All frames of one call are of one kind."""
+    dev = [hasattr(f, "__cuda_array_interface__") for f in frames]
+    if any(dev) and not all(dev):
+        raise ValueError("RGB frames: all host frames or all device frames in one call")
+    if any(dev) and not allow_device:
+        raise ValueError("RGB frames: a host frame is required here")
+    shape = (height, width, 3)
+    out = []
+    for f in frames:
+        if dev and dev[0]:
+            cai = f.__cuda_array_interface__
+            strides = cai.get("strides")
+            if tuple(cai["shape"]) != shape or np.dtype(cai["typestr"]) != np.uint8:
+                raise ValueError("RGB frame: need uint8 of shape %s, got %s %s" % (shape, cai["typestr"], tuple(cai["shape"])))
+            if strides is not None and tuple(strides) != (width * 3, 3, 1):
+                raise ValueError("RGB frame: not C-contiguous (strides %s)" % (tuple(strides),))
+            out.append(int(cai["data"][0]))
+        elif isinstance(f, np.ndarray):
+            if f.dtype != np.uint8 or f.shape != shape or not f.flags["C_CONTIGUOUS"]:
+                raise ValueError("RGB frame: need a C-contiguous uint8 array of shape %s, got %s %s" % (shape, f.dtype, f.shape))
+            out.append(f)
+        elif isinstance(f, (bytes, bytearray)):
+            if len(f) != width * height * 3:
+                raise ValueError("RGB frame: need %d bytes, got %d" % (width * height * 3, len(f)))
+            out.append(np.frombuffer(f, np.uint8))
+        else:
+            raise ValueError("RGB frame: bytes, a uint8 array or an object with __cuda_array_interface__, got %s" % type(f).__name__)
+    return out, (ENC_SRC_DEVICE if dev and dev[0] else 0)
 
 
 def header_decode(jpeg, flags=0):
@@ -424,6 +460,19 @@ class Context:
     # ---- encode -----------------------------------------------------------------------------
     def encode_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None):
         """Encoder.encode_420/422/444 for every raw planar frame (bytes / uint8 arrays) in ``frames``."""
+        return self._encode(frames, None, width, height, chroma, quality, restart_interval, capacity)
+
+    def encode_rgb_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None):
+        """hcj_encode_rgb_batch: every RGB24 frame converted and sub-sampled to ``chroma`` on the device (the stated forward
+        formula, include/hcjpeg.h) and encoded as encode_batch encodes that planar frame.  ``frames``: all host frames
+        (bytes of width*height*3, or C-contiguous uint8 arrays of shape (height, width, 3)) or all device frames (objects
+        with ``__cuda_array_interface__`` of that shape, e.g. torch CUDA tensors, read on the context's stream).
+        Returns (files, status) like encode_batch."""
+        ptrs, flags = _rgb_frames(frames, width, height)
+        return self._encode(ptrs, flags, width, height, chroma, quality, restart_interval, capacity)
+
+    def _encode(self, frames, rgb_flags, width, height, chroma, quality, restart_interval, capacity):
+        """hcj_encode_batch (rgb_flags None) or hcj_encode_rgb_batch with those flags."""
         n = len(frames)
         auto = capacity is None
         if auto:
@@ -434,22 +483,39 @@ class Context:
         caps = (C.c_size_t * max(n, 1))(*([capacity] * n))
         lens = (C.c_size_t * max(n, 1))()
         status = (C.c_int * max(n, 1))()
-        _check(
-            lib().hcj_encode_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, op, caps, lens, status),
-            "hcj_encode_batch",
-        )
+        if rgb_flags is None:
+            _check(
+                lib().hcj_encode_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, op, caps, lens, status),
+                "hcj_encode_batch",
+            )
+        else:
+            _check(
+                lib().hcj_encode_rgb_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, rgb_flags, op, caps,
+                                           lens, status),
+                "hcj_encode_rgb_batch",
+            )
         st = [status[i] for i in range(n)]
         res = [outs[i][: lens[i]].tobytes() if st[i] == 0 else None for i in range(n)]
         # The default capacity is a guess (dense 4:4:4 content at quality 100 exceeds 3 bytes per pixel); the library
         # reports the length a frame needs with HCJ_ERR_BUFFER_TOO_SMALL, so those frames go through once more at that size.
         redo = [i for i in range(n) if st[i] == -30] if auto else []
         if redo:
-            again, st2 = self.encode_batch(
-                [frames[i] for i in redo], width, height, chroma, quality, restart_interval, capacity=max(lens[i] for i in redo)
+            again, st2 = self._encode(
+                [frames[i] for i in redo], rgb_flags, width, height, chroma, quality, restart_interval, max(lens[i] for i in redo)
             )
             for i, o, s2 in zip(redo, again, st2):
                 res[i], st[i] = o, s2
         return res, st
+
+    def rgb_to_yuv(self, frame, width, height, chroma=420):
+        """hcj_rgb_to_yuv: the planar frame (bytes) that encode_rgb_batch encodes for one host RGB24 frame."""
+        (p,), _ = _rgb_frames([frame], width, height, allow_device=False)
+        cw = width if chroma == 444 else width // 2
+        ch = height // 2 if chroma == 420 else height
+        out = np.zeros(width * height + (0 if chroma == 400 else 2 * cw * ch), np.uint8)
+        _check(lib().hcj_rgb_to_yuv(self._h, p if isinstance(p, int) else p.ctypes.data, width, height, chroma, out.ctypes.data, out.size),
+               "hcj_rgb_to_yuv")
+        return out.tobytes()
 
     def encode_quantized(self, frame, width, height, chroma=420, quality=75):
         """Block.quant of every block in encode_seq order (encoder.ml:56-66)."""
