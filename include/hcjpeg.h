@@ -148,6 +148,22 @@ typedef enum hcj_out_mode {
  * segment, and 0xFF fill bytes in front of a marker code are skipped (T.81 B.1.1.2, B.2.4.1, B.2.4.2).  Files the
  * model reads correctly decode identically with and without it. */
 #define HCJ_FLAG_T81_TABLES 2u
+/* Stated extension (the model has no scaled decode): decode at 1/2, 1/4 or 1/8 size, like libjpeg's scale_num /
+ * scale_denom (and Pillow's Image.draft).  Every block of every component is reconstructed straight to k x k samples,
+ * k = 8 / s, with libjpeg's reduced inverse DCTs (jidctred.c: jpeg_idct_4x4, _2x2, _1x1) on the dequantised
+ * coefficients (coefficient x quant entry, natural order, absolute DC), in exact integer arithmetic, output
+ * clamp(x + 128, 0, 255).  Block (bx, by) of component c lands at (bx k, by k) of a padded plane of
+ * decoded_width[c] / s x decoded_height[c] / s.  The frame is then the frame of W' = ceil(width / s) x
+ * H' = ceil(height / s) with the same sampling factors (libjpeg's output size): hcj_frame_info reports width W',
+ * height H', actual_* of that frame, the scaled padded planes and yuv_bytes / planes_bytes / rgb_bytes of those
+ * sizes, while mcus_*, blocks_per_mcu, nblocks and restart_interval keep describing the coded blocks.  Every output
+ * mode works on the scaled planes exactly as on any frame of that size; the coefficient taps are not scaled.
+ * Honoured by hcj_frame_info_get_ex, hcj_decode_batch(_multi), hcj_decode_a_frame, hcj_decode_stream and
+ * hcj_batch_create; hcj_header_decode_ex ignores it.  s = 1 (no bit set) is the ordinary decode. */
+#define HCJ_FLAG_SCALE_1_2 0x10u
+#define HCJ_FLAG_SCALE_1_4 0x20u
+#define HCJ_FLAG_SCALE_1_8 0x30u
+#define HCJ_FLAG_SCALE_MASK 0x30u
 #define HCJ_FLAG_DEFAULT HCJ_FLAG_RESTART_EXT
 
 /* Decoder.decode_a_frame (decoder.ml:422-427) for n independent images; host buffers in and out.

@@ -267,6 +267,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
     sub_log2_env = true;
   }
   const int tile_mcus = HCJ_IDCT_THREADS;  // upper bound on MCUs per IDCT tile (one thread per block)
+  const int scale_log = hcj::scale_log2(flags);  // every image of the batch is decoded at 1 / 2^scale_log (plan_image sizes it)
   // Decoder.Header.decode + the geometry of Decoder.init for every image: independent per image, so spread over
   // a few host threads (it is the serial prologue of every batch: 6 ms single-threaded for 1024 files)
   if (c->hdr_cap < (size_t)std::max(n, 1) * sizeof(hcj_header)) {
@@ -440,7 +441,9 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
       HcjCompGeom &g = d.comp[k];
       g.hs = f.hs[k];
       g.vs = f.vs[k];
-      g.decoded_w = f.decoded_width[k];
+      // The colour kernels read the scratch planes of RGB24 / YUV444 output in 8-byte words: their rows start 8-byte aligned.
+      // Full-size planes are multiples of 8 wide already; scaled ones (8 / s samples per block) get a wider pitch there.
+      g.decoded_w = post_444(mode) ? (int32_t)align_up((size_t)f.decoded_width[k], 8) : f.decoded_width[k];
       g.decoded_h = f.decoded_height[k];
       g.actual_w = f.actual_width[k];
       g.actual_h = f.actual_height[k];
@@ -510,7 +513,8 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
     {
       bool unit_sampling = f.ncomp == 3;
       for (int k = 0; k < f.ncomp; k++) unit_sampling = unit_sampling && f.hs[k] == 1 && f.vs[k] == 1;
-      const bool fusable = mode == HCJ_OUT_RGB24 && f.ncomp == 3 && !d.wide_idct && !getenv("HCJ_NO_FUSED_RGB");
+      // scaled images (HCJ_FLAG_SCALE_*) are never fused: their tiles hold k x k samples per block, K9 converts their planes
+      const bool fusable = mode == HCJ_OUT_RGB24 && f.ncomp == 3 && !d.wide_idct && !scale_log && !getenv("HCJ_NO_FUSED_RGB");
       // sub-sampled: luma 2x2 or 2x1, chroma 1x1, even size (the chroma planes are exactly half)
       const bool sub = f.ncomp == 3 && f.hs[0] == 2 && f.hs[1] == 1 && f.hs[2] == 1 && f.vs[1] == 1 && f.vs[2] == 1 &&
                        ((f.chroma == 420 && f.vs[0] == 2 && f.height % 2 == 0) || (f.chroma == 422 && f.vs[0] == 1)) && f.width % 2 == 0;
@@ -624,6 +628,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
   b->tile_base.assign((size_t)n + 1, 0);
   for (int i = 0; i < n; i++) b->tile_base[i + 1] = b->tile_base[i] + b->descs[i].idct_tiles;
   dv.tile_mcus = tile_mcus;
+  dv.block_k = 8 >> scale_log;
   dv.max_rgb_rows = max_rows;
   dv.max_blocks = max_blocks;
   dv.max_deferred_groups = max_deferred;

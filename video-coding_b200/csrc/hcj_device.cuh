@@ -935,6 +935,118 @@ HCJ_HD void reconstruct_block(const int16_t c[64], const uint16_t q[64], bool fo
 }
 
 // ------------------------------------------------------------------------------------------------
+// Scaled decode (HCJ_FLAG_SCALE_*): libjpeg's reduced inverse DCTs (jidctred.c jpeg_idct_4x4 / _2x2 / _1x1, CONST_BITS
+// 13, PASS1_BITS 2), columns first, then rows, in exact integer arithmetic; out = clamp(x + 128, 0, 255).
+// cw: the block as reconstruct_fast takes it; q: quant table in zig-zag order, plain values.  out[r]: the k samples of
+// row r, packed little-endian.
+// TC is the type of the column pass.  TC = int32_t is exact for blocks the entropy decoders did not flag (quant
+// entries <= 255 and sum(|dequantised coefficient|) = L1 < HCJ_IDCT_L1_LIMIT): every column-pass value is a signed sum
+// of dequantised coefficients of one column with weights of at most 20995 (4x4) / 32768 (2x2), so it stays below
+// 32768 * 60000 + 4096 < 2^31.  The row pass always runs in 64 bits: its inputs can reach 5.2 L1 (4x4) / 4 L1 (2x2),
+// which times its weights overflows 32 bits from L1 of about 20000 / 16000 on.  TC = int64_t (flagged blocks, 16-bit
+// tables) is the reference arithmetic verbatim (DESIGN.md 4).
+// ------------------------------------------------------------------------------------------------
+template <typename T>
+HCJ_HD T dequant_nat(const uint32_t cw[32], const int32_t *q, int n) {  // dequantised coefficient at natural index n
+  const int z = zigzag_forward(n);
+  const int32_t c = (z & 1) ? (int32_t)(int16_t)(cw[z >> 1] >> 16) : (int32_t)(int16_t)(cw[z >> 1] & 0xffffu);
+  return (T)c * (T)q[z];
+}
+
+// One pass of jpeg_idct_4x4 over inputs 0, 1, 2, 3, 5, 6, 7 (input 4 does not contribute), descaled by `sh`.
+template <typename T>
+HCJ_HD void idct4_pass(T c0, T c1, T c2, T c3, T c5, T c6, T c7, int sh, T o[4]) {
+  const T t0 = c0 * (T)(1 << 14);                          // << (CONST_BITS + 1)
+  const T t2 = c2 * (T)15137 - c6 * (T)6270;               // FIX(1.847759065), FIX(0.765366865)
+  const T t10 = t0 + t2, t12 = t0 - t2;
+  const T a0 = c1 * (T)8697 - c3 * (T)17799 + c5 * (T)11893 - c7 * (T)1730;
+  const T a2 = c1 * (T)20995 + c3 * (T)7373 - c5 * (T)4926 - c7 * (T)4176;
+  const T r = (T)1 << (sh - 1);
+  o[0] = (t10 + a2 + r) >> sh;
+  o[1] = (t12 + a0 + r) >> sh;
+  o[2] = (t12 - a0 + r) >> sh;
+  o[3] = (t10 - a2 + r) >> sh;
+}
+
+// One pass of jpeg_idct_2x2 over inputs 0, 1, 3, 5, 7.
+template <typename T>
+HCJ_HD void idct2_pass(T c0, T c1, T c3, T c5, T c7, int sh, T o[2]) {
+  const T t10 = c0 * (T)(1 << 15);                         // << (CONST_BITS + 2)
+  const T t0 = c1 * (T)29692 - c3 * (T)10426 + c5 * (T)6967 - c7 * (T)5906;
+  const T r = (T)1 << (sh - 1);
+  o[0] = (t10 + t0 + r) >> sh;
+  o[1] = (t10 - t0 + r) >> sh;
+}
+
+// A row-pass result + 128, clamped: with TC = int32_t it is below 2^15 in magnitude (see above), so the cast is exact.
+template <typename TC>
+HCJ_HD int32_t reduced_sample(int64_t v) {
+  if (sizeof(TC) == 8) v = v < -128 ? -128 : v > 127 ? 127 : v;
+  return (int32_t)v + 128;
+}
+
+template <typename TC>
+HCJ_HD void reconstruct_4x4(const uint32_t cw[32], const int32_t *q, uint32_t out[4]) {
+  int64_t ws[4][8];
+#pragma unroll
+  for (int c = 0; c < 8; c++) {
+    if (c == 4) continue;  // column 4 is not read by the row pass
+    TC o[4];
+    idct4_pass<TC>(dequant_nat<TC>(cw, q, c), dequant_nat<TC>(cw, q, 8 + c), dequant_nat<TC>(cw, q, 16 + c),
+                   dequant_nat<TC>(cw, q, 24 + c), dequant_nat<TC>(cw, q, 40 + c), dequant_nat<TC>(cw, q, 48 + c),
+                   dequant_nat<TC>(cw, q, 56 + c), 12, o);  // CONST_BITS - PASS1_BITS + 1
+#pragma unroll
+    for (int r = 0; r < 4; r++) ws[r][c] = (int64_t)o[r];
+  }
+#pragma unroll
+  for (int r = 0; r < 4; r++) {
+    int64_t o[4];
+    idct4_pass<int64_t>(ws[r][0], ws[r][1], ws[r][2], ws[r][3], ws[r][5], ws[r][6], ws[r][7], 19, o);  // CONST_BITS + PASS1_BITS + 3 + 1
+    out[r] = pack4_sat(reduced_sample<TC>(o[0]), reduced_sample<TC>(o[1]), reduced_sample<TC>(o[2]), reduced_sample<TC>(o[3]));
+  }
+}
+
+template <typename TC>
+HCJ_HD void reconstruct_2x2(const uint32_t cw[32], const int32_t *q, uint32_t out[2]) {
+  int64_t ws[2][8];
+#pragma unroll
+  for (int c = 1; c < 8; c += 2) {  // columns 1, 3, 5, 7 here, column 0 below; 2, 4, 6 are not read by the row pass
+    TC o[2];
+    idct2_pass<TC>(dequant_nat<TC>(cw, q, c), dequant_nat<TC>(cw, q, 8 + c), dequant_nat<TC>(cw, q, 24 + c),
+                   dequant_nat<TC>(cw, q, 40 + c), dequant_nat<TC>(cw, q, 56 + c), 13, o);  // CONST_BITS - PASS1_BITS + 2
+    ws[0][c] = (int64_t)o[0];
+    ws[1][c] = (int64_t)o[1];
+  }
+  {
+    TC o[2];
+    idct2_pass<TC>(dequant_nat<TC>(cw, q, 0), dequant_nat<TC>(cw, q, 8), dequant_nat<TC>(cw, q, 24), dequant_nat<TC>(cw, q, 40),
+                   dequant_nat<TC>(cw, q, 56), 13, o);
+    ws[0][0] = (int64_t)o[0];
+    ws[1][0] = (int64_t)o[1];
+  }
+#pragma unroll
+  for (int r = 0; r < 2; r++) {
+    int64_t o[2];
+    idct2_pass<int64_t>(ws[r][0], ws[r][1], ws[r][3], ws[r][5], ws[r][7], 20, o);  // CONST_BITS + PASS1_BITS + 3 + 2
+    out[r] = pack4_sat(reduced_sample<TC>(o[0]), reduced_sample<TC>(o[1]), 0, 0);
+  }
+}
+
+// jpeg_idct_1x1: DESCALE(dc * q, 3).  Exact in 32 bits for any int16 DC and 16-bit quant entry (|dc q| + 4 < 2^31).
+HCJ_HD uint32_t reconstruct_1x1(uint32_t cw0, int32_t q0) {
+  const int32_t d = (int32_t)(int16_t)(cw0 & 0xffffu) * q0;
+  return pack4_sat(((d + 4) >> 3) + 128, 0, 0, 0);
+}
+
+// The whole scaled reconstruction of one block as the IDCT kernel selects it (wide: the block is flagged or the image
+// has quant entries above 255).  k = 4, 2, 1; out[r] as above.
+HCJ_HD void reconstruct_scaled(const uint32_t cw[32], const int32_t *q, int k, bool wide, uint32_t *out) {
+  if (k == 1) out[0] = reconstruct_1x1(cw[0], q[0]);
+  else if (k == 2) wide ? reconstruct_2x2<int64_t>(cw, q, out) : reconstruct_2x2<int32_t>(cw, q, out);
+  else wide ? reconstruct_4x4<int64_t>(cw, q, out) : reconstruct_4x4<int32_t>(cw, q, out);
+}
+
+// ------------------------------------------------------------------------------------------------
 // Dct.Chen.forward_8x8 (dct.ml:109-196): columns first, then rows.  Inputs are pixel - 128, so 32-bit
 // arithmetic is exact (|value| < 2^21 throughout).
 // ------------------------------------------------------------------------------------------------

@@ -332,6 +332,20 @@ int plan_image(const hcj_header &h, unsigned flags, ImagePlan *plan) {
     if (f.mcus_wide * f.hs[i] * 8 > f.decoded_width[i] || f.mcus_high * f.vs[i] * 8 > f.decoded_height[i])
       return HCJ_ERR_PLANE_BOUNDS;
   f.restart_interval = ((flags & HCJ_FLAG_RESTART_EXT) && h.has_restart_interval) ? h.restart_interval : 0;
+  // Scaled decode (HCJ_FLAG_SCALE_*): the frame of ceil(w / s) x ceil(h / s) with the same sampling factors, padded
+  // planes of decoded_* / s (multiples of 8 / s: they hold every block's k x k samples); the block geometry above stays.
+  const int scale_log = hcj::scale_log2(flags);
+  if (scale_log) {
+    const int s = 1 << scale_log;
+    f.width = (h.width + s - 1) >> scale_log;
+    f.height = (h.height + s - 1) >> scale_log;
+    for (int i = 0; i < ncomp; i++) {
+      f.decoded_width[i] >>= scale_log;
+      f.decoded_height[i] >>= scale_log;
+      f.actual_width[i] = (int)((int64_t)f.width * f.hs[i] / max_h);
+      f.actual_height[i] = (int)((int64_t)f.height * f.vs[i] / max_v);
+    }
+  }
   f.planes_bytes = 0;
   for (int i = 0; i < ncomp; i++) f.planes_bytes += (size_t)f.decoded_width[i] * f.decoded_height[i];
   // get_yuv_frame -> Frame.of_planes -> infer_chroma_subsampling (frame.ml:42-61)

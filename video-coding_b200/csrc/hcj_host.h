@@ -30,6 +30,8 @@ struct ImagePlan {
   int blk_comp[HCJ_MAX_BPM], blk_bx[HCJ_MAX_BPM], blk_by[HCJ_MAX_BPM];
 };
 int plan_image(const hcj_header &h, unsigned flags, ImagePlan *plan);
+// HCJ_FLAG_SCALE_*: log2 of the scale denominator s (0 = full size, 1..3 = 1/2, 1/4, 1/8)
+inline int scale_log2(unsigned flags) { return (int)((flags & HCJ_FLAG_SCALE_MASK) >> 4); }
 
 // Tables.Specification.create_code_table + Tables.Lut.create (tables.ml:27-51,478-502), re-packed as
 // a HCJ_LUT_BITS primary table plus the model's full 2^max_bits table.

@@ -1582,6 +1582,64 @@ __device__ __noinline__ void wide_block_store_staged(const uint4 *tile, int slot
   store_block_rows(pix, dst, stride, x, y, w_limit, h_limit);
 }
 
+// Scaled decode (HCJ_FLAG_SCALE_*): k x k samples (k = 4, 2, 1) of a block at (x, y) of its scaled plane, cropped like
+// store_block_rows.  pix[r]: row r, packed.  With k = 4 a warp's 32 horizontally adjacent blocks write 128 contiguous bytes.
+template <int K>
+__device__ __forceinline__ void store_block_rows_k(const uint32_t *pix, uint8_t *dst, int stride, int x, int y, int w_limit,
+                                                   int h_limit) {
+  uint8_t *row = dst + (size_t)y * stride + x;
+  const bool fast = (x + K <= w_limit) && (((uintptr_t)row & (K - 1)) == 0) && ((stride & (K - 1)) == 0);
+#pragma unroll
+  for (int r = 0; r < K; r++) {
+    if (y + r >= h_limit) break;
+    uint8_t *p = row + (size_t)r * stride;
+    if (fast) {
+      if (K == 4) *reinterpret_cast<uint32_t *>(p) = pix[r];
+      else if (K == 2) *reinterpret_cast<uint16_t *>(p) = (uint16_t)pix[r];
+      else *p = (uint8_t)pix[r];
+    } else {
+#pragma unroll
+      for (int i = 0; i < K; i++)
+        if (x + i < w_limit) p[i] = (uint8_t)(pix[r] >> (8 * i));
+    }
+  }
+}
+
+// Flagged blocks and 16-bit tables: the 64-bit column pass, out of line like wide_block_store_staged.
+template <int K>
+__device__ __noinline__ void scaled_block_store_wide(const uint4 *tile, int slot, const int32_t *q, uint8_t *dst, int stride, int x,
+                                                     int y, int h_limit) {
+  uint32_t cw[32], pix[K];
+  for (int j = 0; j < 8; j++) {
+    const uint4 u = tile[slot * 8 + (j ^ (slot & 7))];
+    cw[4 * j] = u.x, cw[4 * j + 1] = u.y, cw[4 * j + 2] = u.z, cw[4 * j + 3] = u.w;
+  }
+  reconstruct_scaled(cw, q, K, true, pix);
+  store_block_rows_k<K>(pix, dst, stride, x, y, stride, h_limit);
+}
+
+// One block of the staged tile reconstructed at 1/s (K = 8 / s) and stored.  K = 1 reads only the DC word.
+template <int K>
+__device__ __forceinline__ void scaled_block_store(const uint4 *tile, int slot, const int32_t *q, bool wide, uint8_t *dst, int stride,
+                                                   int x, int y, int h_limit) {
+  uint32_t pix[K];
+  if (K == 1) {
+    pix[0] = reconstruct_1x1(tile[slot * 8 + (slot & 7)].x, q[0]);  // chunk 0 of the block sits at chunk slot & 7 of its row
+  } else if (wide) {
+    scaled_block_store_wide<K>(tile, slot, q, dst, stride, x, y, h_limit);
+    return;
+  } else {
+    uint32_t cw[32];
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+      const uint4 u = tile[slot * 8 + (j ^ (slot & 7))];
+      cw[4 * j] = u.x, cw[4 * j + 1] = u.y, cw[4 * j + 2] = u.z, cw[4 * j + 3] = u.w;
+    }
+    reconstruct_scaled(cw, q, K, false, pix);
+  }
+  store_block_rows_k<K>(pix, dst, stride, x, y, stride, h_limit);
+}
+
 // Persistent CTAs (HCJ_IDCT_CTAS_PER_SM per SM): each owns a contiguous range of the batch's tiles and keeps the coefficient
 // tile, the quant tables and the wide-block flags of tile i+1 in flight (cp.async) while tile i is being
 // transformed.  The thread -> block mapping depends only on (image geometry, tile width): it is computed
@@ -2011,7 +2069,9 @@ __device__ __forceinline__ void idct_tile_rgb_sub(const DecodeBatchDev &b, const
 
 // FUSED = true is the instance launched for RGB24 batches that hold 4:4:4 images: their tiles take the fused path
 // (idct_tile_rgb444 below); every other tile, and every tile of the FUSED = false instance, takes the planar path.
-template <bool FUSED>
+// K: samples per block side in the output planes; K = 4, 2, 1 are the scaled decodes (HCJ_FLAG_SCALE_*, never fused),
+// which keep the tile plan, the staging and the thread -> block mapping and change only the transform and the store.
+template <bool FUSED, int K = 8>
 __global__ void __launch_bounds__(IDCT_MAX_THREADS, HCJ_IDCT_CTAS_PER_SM)
     k_idct_persistent(const __grid_constant__ DecodeBatchDev b, int mode) {
   extern __shared__ uint4 s_dyn[];
@@ -2063,9 +2123,9 @@ __global__ void __launch_bounds__(IDCT_MAX_THREADS, HCJ_IDCT_CTAS_PER_SM)
       const uint32_t slot = (uint32_t)(m * d.bpm + g.first_blk + by * g.hs + bx);
       const bool mine = tid < (int)t.nblk;
       IdctMap mp;
-      mp.xy = (uint32_t)(m * g.hs * 8 + bx * 8) | (uint32_t)(by * 8) << 16;
+      mp.xy = (uint32_t)(m * g.hs * K + bx * K) | (uint32_t)(by * K) << 16;
       mp.misc = (mine ? slot : 0u) | (uint32_t)c << 8 | (mine ? 1u << 10 : 0u) | (d.wide_idct ? 1u << 11 : 0u) |
-                (uint32_t)(g.hs * 8) << 12 | (uint32_t)(g.vs * 8) << 18;
+                (uint32_t)(g.hs * K) << 12 | (uint32_t)(g.vs * K) << 18;
       if (mode == 0) {
         mp.plane = b.out + d.out_off + g.out_off;
         mp.stride = g.actual_w;
@@ -2088,7 +2148,14 @@ __global__ void __launch_bounds__(IDCT_MAX_THREADS, HCJ_IDCT_CTAS_PER_SM)
       idct_tile_rgb444(b, t, st, mp, tnow);
     } else if (FUSED && t.fused == 2u) {
       idct_tile_rgb_sub(b, t, st, mp, tnow);
-    } else if (mp.misc & (1u << 10)) {
+    } else if (K != 8 && (mp.misc & (1u << 10))) {
+      const int slot = (int)(mp.misc & 255u);
+      const uint32_t fbit = (uint32_t)(t.blk0 & 127u) + slot;
+      const bool wide = (mp.misc & (1u << 11)) || ((reinterpret_cast<const uint32_t *>(st.flags)[fbit >> 5] >> (fbit & 31u)) & 1u);
+      const int x = (int)t.m0 * (int)((mp.misc >> 12) & 63u) + (int)(mp.xy & 0xffffu);
+      const int y = (int)t.my * (int)((mp.misc >> 18) & 63u) + (int)(mp.xy >> 16);
+      scaled_block_store<K>(st.tile, slot, st.q + ((mp.misc >> 8) & 3u) * 128u, wide, mp.plane, mp.stride, x, y, mp.h_limit);
+    } else if (K == 8 && (mp.misc & (1u << 10))) {
       const int slot = (int)(mp.misc & 255u);
       uint32_t cw[32];
 #pragma unroll
@@ -2125,7 +2192,10 @@ void launch_idct(const DecodeBatchDev &b, int mode, cudaStream_t s) {
   k_idct_plan<<<dim3((b.max_idct_tiles + 127) / 128, b.img_hi - b.img_lo), 128, 0, s>>>(b);
   const uint32_t total = b.tile_hi - b.tile_lo;
   const unsigned ctas = (unsigned)(total < (uint32_t)grid ? total : grid);
-  if (mode == 2 && (b.has_fused || b.has_fused_sub)) k_idct_persistent<true><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  if (b.block_k == 4) k_idct_persistent<false, 4><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  else if (b.block_k == 2) k_idct_persistent<false, 2><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  else if (b.block_k == 1) k_idct_persistent<false, 1><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  else if (mode == 2 && (b.has_fused || b.has_fused_sub)) k_idct_persistent<true><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
   else k_idct_persistent<false><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
 }
 
@@ -2701,6 +2771,9 @@ int configure_device(int *sm_count) {
                              (int)(base + (SPEC_WRITE_THREADS / 32) * HR_STAGE_WORDS * sizeof(uint32_t)));
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
   if (sm_count) *sm_count = sms;
   return (int)e;
 }

@@ -58,6 +58,7 @@ struct DecodeBatchDev {
   uint32_t total_idct_tiles;
   uint32_t tile_lo, tile_hi;      // tiles of the images [img_lo, img_hi)
   int tile_mcus;                  // MCUs per IDCT tile (upper bound; per-image value derived in-kernel)
+  int block_k;                    // samples per block side in the output planes: 8, or 8 / s for a scaled decode (HCJ_FLAG_SCALE_*)
   uint32_t max_rgb_rows;          // max image height (RGB mode)
   int has_444, has_subsampled;    // the batch holds 4:4:4 / sub-sampled images that go through k_rgb: which instances to launch
                                   // (has_subsampled: bit 0 = of even size, bit 1 = of odd size)

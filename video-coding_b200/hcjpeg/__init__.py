@@ -22,6 +22,12 @@ OUT_YUV, OUT_PLANES, OUT_RGB24, OUT_YUV444 = 0, 1, 2, 3
 FLAG_RESTART_EXT = 1
 FLAG_T81_TABLES = 2
 FLAG_DEFAULT = FLAG_RESTART_EXT
+# Scaled decode (stated extension, include/hcjpeg.h): OR one of these into the decode flags to decode at 1/2, 1/4 or 1/8
+# size with libjpeg's reduced IDCTs (what Pillow's Image.draft gives); frame_info(jpeg, flags) reports the scaled frame.
+FLAG_SCALE_1_2 = 0x10
+FLAG_SCALE_1_4 = 0x20
+FLAG_SCALE_1_8 = 0x30
+FLAG_SCALE_MASK = 0x30
 ENC_SRC_DEVICE = 1  # hcj_encode_rgb_batch: the frames are device pointers on the context's device
 
 MAX_COMPONENTS = 4
@@ -339,7 +345,8 @@ def header_decode(jpeg, flags=0):
 
 
 def frame_info(jpeg, flags=FLAG_DEFAULT):
-    """Geometry fixed by Decoder.init (decoder.ml:304-345)."""
+    """Geometry fixed by Decoder.init (decoder.ml:304-345).  With FLAG_SCALE_* in ``flags``: the scaled frame (width,
+    height, planes and output sizes of the 1/s decode; the block geometry stays that of the file)."""
     f = FrameInfo()
     _check(lib().hcj_frame_info_get_ex(jpeg, len(jpeg), flags, C.byref(f)), "Decoder.init")
     return f
@@ -397,7 +404,8 @@ class Context:
     # ---- decode -----------------------------------------------------------------------------
     def decode_batch(self, jpegs, mode=OUT_YUV, flags=FLAG_DEFAULT, raise_on_error=False):
         """Decoder.decode_a_frame for every element of ``jpegs`` (bytes).  Returns (outputs, status):
-        outputs[i] is a uint8 array (None where status[i] != 0)."""
+        outputs[i] is a uint8 array (None where status[i] != 0).  Outputs are sized by frame_info(jpeg, flags), so a
+        FLAG_SCALE_* in ``flags`` (here and in every decode entry point) gives the scaled frames."""
         n = len(jpegs)
         infos, caps, outs = [], [], []
         for j in jpegs:
