@@ -164,6 +164,29 @@ typedef enum hcj_out_mode {
 #define HCJ_FLAG_SCALE_1_4 0x20u
 #define HCJ_FLAG_SCALE_1_8 0x30u
 #define HCJ_FLAG_SCALE_MASK 0x30u
+/* Stated extension (the model reconstructs with Chen-Wang and Planar_444): reconstruct samples as libjpeg-turbo's default
+ * decompressor does (dct_method JDCT_ISLOW, do_fancy_upsampling TRUE; its C code paths are the specification), so that
+ * RGB24 equals what Pillow, OpenCV and torchvision's CPU decoder give.
+ *  - Every block of every component, in every output mode: jidctint.c jpeg_idct_islow on the dequantised coefficients
+ *    (coefficient x quant entry, natural order, absolute DC), columns first, 64-bit intermediates, column-pass results
+ *    truncated to 32 bits, row pass descaled by 18, then libjpeg's range-limit table with its wrap:
+ *    clamp(((v + 512) & 1023) - 512 + 128, 0, 255).
+ *  - HCJ_OUT_RGB24 / HCJ_OUT_YUV444: jdsample.c up-sampling of each component's real plane, ceil(W h_c / h_max) x
+ *    ceil(H v_c / v_max) samples, by (h_max / h_c, v_max / v_c): (1, 1) copy; (2, 1) / (2, 2) / (1, 2) the fancy
+ *    (triangle) filters h2v1 / h2v2 / h1v2, edges replicated, (2, 1) and (2, 2) plain replication when the real plane is
+ *    at most 2 samples wide; any other integral ratio replication (int_upsample); a non-integral ratio is
+ *    HCJ_ERR_UNSUPPORTED_GEOMETRY.  Cropped to W x H; colour as without the flag (the formula is jdcolor.c's).
+ *    RGB24 equals Image.open(f).convert("RGB"), YUV444 Image.draft("YCbCr", size).
+ *  - HCJ_OUT_YUV / HCJ_OUT_PLANES keep their layout and the model's crop rules, with islow samples.
+ *  - hcj_frame_info is unchanged except that a 3-component frame with chroma 0 but integral ratios (4:4:0, 4:1:1)
+ *    reports rgb_bytes = W H 3 and decodes to RGB24 / YUV444.  4-component frames give HCJ_ERR_UNSUPPORTED_GEOMETRY in
+ *    RGB24 / YUV444 (libjpeg would take them as CMYK / YCCK); fewer than 3 components keep HCJ_ERR_NEED_3_COMPONENTS.
+ *  - Honoured by hcj_frame_info_get_ex, hcj_decode_batch(_multi), hcj_decode_a_frame, hcj_decode_stream and
+ *    hcj_batch_create; hcj_header_decode_ex and the debug taps (coefficients, entropy, block log, hcj_idct_blocks)
+ *    ignore it.  Together with an HCJ_FLAG_SCALE_* bit it is HCJ_ERR_INVALID_ARG.
+ * libjpeg-turbo's x86 SIMD IDCT works in 16-bit lanes and differs from its C code on blocks whose dequantised
+ * coefficients do not fit 16 bits; this flag follows the C code there. */
+#define HCJ_FLAG_LIBJPEG 0x40u
 #define HCJ_FLAG_DEFAULT HCJ_FLAG_RESTART_EXT
 
 /* Decoder.decode_a_frame (decoder.ml:422-427) for n independent images; host buffers in and out.

@@ -225,7 +225,9 @@ static cudaError_t upload_files(const hcj_batch *b, const uint8_t *const *jpeg, 
 
 static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *len, int n, int mode, unsigned flags,
                         int *status, hcj_batch **out, bool with_files) {
-  if (!c || !out || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!jpeg || !len)) || mode < 0 || mode > HCJ_OUT_YUV444) return HCJ_ERR_INVALID_ARG;
+  if (!c || !out || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!jpeg || !len)) || mode < 0 || mode > HCJ_OUT_YUV444 ||
+      ((flags & HCJ_FLAG_LIBJPEG) && (flags & HCJ_FLAG_SCALE_MASK)))
+    return HCJ_ERR_INVALID_ARG;
   *out = nullptr;
   CU_TRY(cudaSetDevice(c->device));
   hcj_batch *b = new (std::nothrow) hcj_batch;
@@ -268,6 +270,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
   }
   const int tile_mcus = HCJ_IDCT_THREADS;  // upper bound on MCUs per IDCT tile (one thread per block)
   const int scale_log = hcj::scale_log2(flags);  // every image of the batch is decoded at 1 / 2^scale_log (plan_image sizes it)
+  const bool libjpeg = (flags & HCJ_FLAG_LIBJPEG) != 0;  // every image of the batch is reconstructed as libjpeg does
   // Decoder.Header.decode + the geometry of Decoder.init for every image: independent per image, so spread over
   // a few host threads (it is the serial prologue of every batch: 6 ms single-threaded for 1024 files)
   if (c->hdr_cap < (size_t)std::max(n, 1) * sizeof(hcj_header)) {
@@ -393,6 +396,8 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
     }
     if (st == HCJ_OK && (mode == HCJ_OUT_YUV || post_444(mode))) {
       if (f.ncomp < 3) st = HCJ_ERR_NEED_3_COMPONENTS;  // decoder.ml:415-420
+      // jdsample.c: integral ratios of 3-component frames (4-component ones would be CMYK / YCCK to libjpeg)
+      else if (libjpeg && post_444(mode)) st = f.ncomp == 3 && plan.up_integral ? HCJ_OK : HCJ_ERR_UNSUPPORTED_GEOMETRY;
       else if (f.chroma == 0) st = HCJ_ERR_FRAME_INFER;  // frame.ml:44,55
     }
     b->host_status[i] = st;
@@ -450,6 +455,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
       g.pair = pair_of[k];
       g.qt = k;
       g.first_blk = first_blk;
+      if (libjpeg && post_444(mode)) g.up_h = (uint8_t)plan.up_h[k], g.up_v = (uint8_t)plan.up_v[k];
       first_blk += g.hs * g.vs;
       g.plane_off = (post_444(mode) ? plane_total : 0) + plane_acc;
       plane_acc += (size_t)g.decoded_w * g.decoded_h;
@@ -514,7 +520,8 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
       bool unit_sampling = f.ncomp == 3;
       for (int k = 0; k < f.ncomp; k++) unit_sampling = unit_sampling && f.hs[k] == 1 && f.vs[k] == 1;
       // scaled images (HCJ_FLAG_SCALE_*) are never fused: their tiles hold k x k samples per block, K9 converts their planes
-      const bool fusable = mode == HCJ_OUT_RGB24 && f.ncomp == 3 && !d.wide_idct && !scale_log && !getenv("HCJ_NO_FUSED_RGB");
+      // nor are libjpeg reconstructions (HCJ_FLAG_LIBJPEG): the fused tiles hold the model's transform
+      const bool fusable = mode == HCJ_OUT_RGB24 && f.ncomp == 3 && !d.wide_idct && !scale_log && !libjpeg && !getenv("HCJ_NO_FUSED_RGB");
       // sub-sampled: luma 2x2 or 2x1, chroma 1x1, even size (the chroma planes are exactly half)
       const bool sub = f.ncomp == 3 && f.hs[0] == 2 && f.hs[1] == 1 && f.hs[2] == 1 && f.vs[1] == 1 && f.vs[2] == 1 &&
                        ((f.chroma == 420 && f.vs[0] == 2 && f.height % 2 == 0) || (f.chroma == 422 && f.vs[0] == 1)) && f.width % 2 == 0;
@@ -534,7 +541,8 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
       const uint32_t def_rows = f.vs[0] == 2 ? (uint32_t)(f.actual_height[1] - 1) / 8 : 0;
       max_deferred = std::max(max_deferred, def_rows * (((uint32_t)f.width + 15) / 16) + (tpr - 1) * (uint32_t)f.height);
     }
-    else if (f.chroma == 444) b->dev.has_444 = 1;
+    else if (f.chroma == 444) b->dev.has_444 = 1;  // 4:4:4 needs no up-sampling: libjpeg's copy is Planar_444's
+    else if (libjpeg && post_444(mode)) d.libjpeg = 1, b->dev.has_libjpeg = 1;
     else b->dev.has_subsampled |= ((f.width & 1) || (f.chroma == 420 && (f.height & 1))) ? 2 : 1;
     max_blocks = std::max(max_blocks, d.nblocks);
     max_width = std::max(max_width, (uint32_t)f.width);
@@ -629,6 +637,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
   for (int i = 0; i < n; i++) b->tile_base[i + 1] = b->tile_base[i] + b->descs[i].idct_tiles;
   dv.tile_mcus = tile_mcus;
   dv.block_k = 8 >> scale_log;
+  dv.islow = libjpeg ? 1 : 0;
   dv.max_rgb_rows = max_rows;
   dv.max_blocks = max_blocks;
   dv.max_deferred_groups = max_deferred;
@@ -642,7 +651,7 @@ static int batch_create(hcj_ctx *c, const uint8_t *const *jpeg, const size_t *le
   dv.ls_hi = (uint32_t)list_spec.size();
   b->list_restart = list_restart;
   b->list_spec = list_spec;
-  b->kernels = hcjk::destuff_kernel_count() + (dv.n_restart ? 1 : 0) + (dv.n_spec ? hcjk::huff_spec_kernel_count(dv) : 0) + hcjk::idct_kernel_count() + (post_444(mode) ? dv.has_444 + (mode == HCJ_OUT_RGB24 ? (dv.has_subsampled & 1) + (dv.has_subsampled >> 1) + dv.has_fused + dv.has_fused_sub : (dv.has_subsampled ? 1 : 0)) : 0);
+  b->kernels = hcjk::destuff_kernel_count() + (dv.n_restart ? 1 : 0) + (dv.n_spec ? hcjk::huff_spec_kernel_count(dv) : 0) + hcjk::idct_kernel_count() + (post_444(mode) ? dv.has_444 + (mode == HCJ_OUT_RGB24 ? (dv.has_subsampled & 1) + (dv.has_subsampled >> 1) + dv.has_fused + dv.has_fused_sub : (dv.has_subsampled ? 1 : 0)) + dv.has_libjpeg : 0);
 
   // ---- upload
   cudaStream_t s = c->stream;

@@ -58,7 +58,8 @@ struct HcjCompGeom {
   int32_t pair;                   // index into the table set
   int32_t qt;                     // index into the image's quant tables (qt_off + 64 * qt)
   int32_t first_blk;              // first block-in-MCU index of this component
-  int32_t pad_;
+  uint8_t up_h, up_v;             // HCJ_FLAG_LIBJPEG, RGB24 / YUV444: up-sampling ratios h_max / h_c, v_max / v_c
+  uint16_t pad_;
   uint64_t plane_off;             // byte offset of the padded plane in the batch plane buffer
   uint64_t out_off;               // byte offset of this component's plane in the image's output
 };
@@ -86,7 +87,7 @@ struct HcjImageDesc {
   uint8_t wide_idct;     // 1: some quant entry > 255 -> always take the 64-bit IDCT
   uint8_t valid;         // 0: header/geometry failed on the host; kernels skip the image
   uint8_t fused_rgb;     // RGB24 output, no 16-bit quant entries: k_idct_persistent converts to RGB itself (1 = 4:4:4, 2 = 4:2:0 / 4:2:2 of even size)
-  uint8_t pad_[1];
+  uint8_t libjpeg;       // HCJ_FLAG_LIBJPEG, RGB24 / YUV444, not 4:4:4: k_rgb_libjpeg up-samples it (comp[].up_h / up_v)
   uint32_t table_set;    // index into the batch table sets
   uint32_t qt_off;       // offset (uint16 entries) of this image's quant tables [nqt][64], zig-zag order
   // output

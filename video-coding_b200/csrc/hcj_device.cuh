@@ -1047,6 +1047,101 @@ HCJ_HD void reconstruct_scaled(const uint32_t cw[32], const int32_t *q, int k, b
 }
 
 // ------------------------------------------------------------------------------------------------
+// libjpeg reconstruction (HCJ_FLAG_LIBJPEG): jidctint.c jpeg_idct_islow (CONST_BITS 13, PASS1_BITS 2), columns first,
+// on the dequantised coefficients.  The column pass's results are stored as C int (truncated to 32 bits); the row
+// pass's, descaled by 18, index libjpeg's range-limit table: sample = clamp(((v + 512) & 1023) - 512 + 128, 0, 255).
+// That depends on bits 0..27 of the row pass's sum only, so the row pass is exact in wrapping 32-bit arithmetic for
+// every block.  The column pass is exact in wrapping 32-bit arithmetic when its sums fit 32 bits: for blocks the
+// entropy decoders did not flag (quant entries <= 255, sum(|dequantised coefficient|) = L1 < HCJ_IDCT_L1_LIMIT) they
+// are at most 11363 L1 + 1024 < 2^30 (DESIGN.md 4).  Flagged blocks and 16-bit tables take the column pass in 64 bits
+// (islow_wide).  T = uint32_t is the wrapping arithmetic, T = int64_t the C code's JLONG.
+// ------------------------------------------------------------------------------------------------
+// One islow pass over inputs c0..c7 (the even part, then the odd part of jidctint.c), before the descale.
+template <typename T>
+HCJ_HD void islow_pass(T c0, T c1, T c2, T c3, T c4, T c5, T c6, T c7, T o[8]) {
+  const T z1 = (c2 + c6) * (T)4433;                                  // FIX_0_541196100
+  const T t2 = z1 + c6 * (T)-15137, t3 = z1 + c2 * (T)6270;          // FIX_1_847759065, FIX_0_765366865
+  const T t0 = (c0 + c4) * (T)8192, t1 = (c0 - c4) * (T)8192;       // << CONST_BITS
+  const T t10 = t0 + t3, t13 = t0 - t3, t11 = t1 + t2, t12 = t1 - t2;
+  const T z5 = (c7 + c3 + c5 + c1) * (T)9633;                        // FIX_1_175875602
+  const T za = (c7 + c1) * (T)-7373, zb = (c5 + c3) * (T)-20995;     // FIX_0_899976223, FIX_2_562915447
+  const T zc = (c7 + c3) * (T)-16069 + z5, zd = (c5 + c1) * (T)-3196 + z5;  // FIX_1_961570560, FIX_0_390180644
+  const T p0 = c7 * (T)2446 + za + zc, p1 = c5 * (T)16819 + zb + zd;  // FIX_0_298631336, FIX_2_053119869
+  const T p2 = c3 * (T)25172 + zb + zc, p3 = c1 * (T)12299 + za + zd; // FIX_3_072711738, FIX_1_501321110
+  o[0] = t10 + p3, o[7] = t10 - p3, o[1] = t11 + p2, o[6] = t11 - p2;
+  o[2] = t12 + p1, o[5] = t12 - p1, o[3] = t13 + p0, o[4] = t13 - p0;
+}
+
+// DESCALE(x, CONST_BITS - PASS1_BITS) stored as C int.
+HCJ_HD int32_t islow_ws(uint32_t v) { return (int32_t)(v + 1024u) >> 11; }
+HCJ_HD int32_t islow_ws(int64_t v) { return (int32_t)((v + 1024) >> 11); }
+// range_limit[DESCALE(x, CONST_BITS + PASS1_BITS + 3) & RANGE_MASK] before the final clamp (pack4_sat): adding 2^27
+// moves the wrap point of the 10-bit index from 0 to -512.
+HCJ_HD int32_t islow_sample(uint32_t v) { return (int32_t)(((v + (1u << 17) + (1u << 27)) >> 18) & 1023u) - 384; }
+
+// Row pass of the islow block ws[64] (natural order, C int), packed into out[2r], out[2r + 1] as reconstruct_fast.
+HCJ_HD void islow_rows(const int32_t ws[64], uint32_t out[16]) {
+#pragma unroll
+  for (int r = 0; r < 8; r++) {
+    const int32_t *w = ws + 8 * r;
+    uint32_t o[8];
+    islow_pass<uint32_t>(w[0], w[1], w[2], w[3], w[4], w[5], w[6], w[7], o);
+    out[2 * r] = pack4_sat(islow_sample(o[0]), islow_sample(o[1]), islow_sample(o[2]), islow_sample(o[3]));
+    out[2 * r + 1] = pack4_sat(islow_sample(o[4]), islow_sample(o[5]), islow_sample(o[6]), islow_sample(o[7]));
+  }
+}
+
+// Unflagged blocks, quant entries <= 255: the table in dp2a form (HCJ_QD), as reconstruct_fast takes it.
+HCJ_HD void islow_fast(const uint32_t cw[32], const int32_t *__restrict__ qd, uint32_t out[16]) {
+  int32_t v[64];
+#pragma unroll
+  for (int j = 0; j < 32; j++) {
+    v[zigzag_inverse(2 * j)] = dequant_lo(cw[j], qd[2 * j]);
+    v[zigzag_inverse(2 * j + 1)] = dequant_hi(cw[j], qd[2 * j + 1]);
+  }
+#pragma unroll
+  for (int c = 0; c < 8; c++) {
+    uint32_t o[8];
+    islow_pass<uint32_t>(v[c], v[8 + c], v[16 + c], v[24 + c], v[32 + c], v[40 + c], v[48 + c], v[56 + c], o);
+#pragma unroll
+    for (int r = 0; r < 8; r++) v[8 * r + c] = islow_ws(o[r]);
+  }
+  islow_rows(v, out);
+}
+
+// Any block, any 16-bit table: q plain, zig-zag order.  The column pass is jidctint.c's JLONG arithmetic verbatim.
+HCJ_HD void islow_wide(const uint32_t *cw, const int32_t *q, uint32_t *out) {
+  int32_t ws[64];
+  for (int c = 0; c < 8; c++) {
+    int64_t o[8];
+    islow_pass<int64_t>(dequant_nat<int64_t>(cw, q, c), dequant_nat<int64_t>(cw, q, 8 + c), dequant_nat<int64_t>(cw, q, 16 + c),
+                        dequant_nat<int64_t>(cw, q, 24 + c), dequant_nat<int64_t>(cw, q, 32 + c), dequant_nat<int64_t>(cw, q, 40 + c),
+                        dequant_nat<int64_t>(cw, q, 48 + c), dequant_nat<int64_t>(cw, q, 56 + c), o);
+    for (int r = 0; r < 8; r++) ws[8 * r + c] = islow_ws(o[r]);
+  }
+  islow_rows(ws, out);
+}
+
+// libjpeg's up-sampling (jdsample.c, do_fancy_upsampling) of one component to output sample (x, y).  p: the component's
+// plane (pitch bytes per row) of which rw x rh samples are real (ceil(W / hr) x ceil(H / vr)); (hr, vr) = (h_max / h_c,
+// v_max / v_c).  The fancy filters clamp their neighbours to the real plane, which gives libjpeg's edge columns and
+// its replicated context rows.  h2v1 / h2v2 replicate instead when the real plane is at most 2 samples wide.
+HCJ_HD int libjpeg_upsample(const uint8_t *p, int pitch, int rw, int rh, int hr, int vr, int x, int y) {
+  const int j = x / hr, i = y / vr;
+  int jn = j + ((x & 1) ? 1 : -1), ni = i + ((y & 1) ? 1 : -1);
+  jn = jn < 0 ? 0 : jn > rw - 1 ? rw - 1 : jn;
+  ni = ni < 0 ? 0 : ni > rh - 1 ? rh - 1 : ni;
+  const int a = p[(int64_t)i * pitch + j];
+  if (hr == 1 && vr == 2) return (3 * a + p[(int64_t)ni * pitch + j] + 1 + (y & 1)) >> 2;           // h1v2_fancy_upsample
+  if (hr == 2 && vr == 1 && rw > 2) return (3 * a + p[(int64_t)i * pitch + jn] + 1 + (x & 1)) >> 2;  // h2v1_fancy_upsample
+  if (hr == 2 && vr == 2 && rw > 2) {                                                             // h2v2_fancy_upsample
+    const int cs = 3 * a + p[(int64_t)ni * pitch + j], cn = 3 * p[(int64_t)i * pitch + jn] + p[(int64_t)ni * pitch + jn];
+    return (3 * cs + cn + 8 - (x & 1)) >> 4;
+  }
+  return a;  // fullsize_upsample, h2v1 / h2v2_upsample, int_upsample
+}
+
+// ------------------------------------------------------------------------------------------------
 // Dct.Chen.forward_8x8 (dct.ml:109-196): columns first, then rows.  Inputs are pixel - 128, so 32-bit
 // arithmetic is exact (|value| < 2^21 throughout).
 // ------------------------------------------------------------------------------------------------

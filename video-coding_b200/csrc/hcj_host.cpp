@@ -263,8 +263,10 @@ int mjpeg_split(const uint8_t *s, size_t len, size_t *offsets, size_t *lengths, 
 int plan_image(const hcj_header &h, unsigned flags, ImagePlan *plan) {
   memset(plan, 0, sizeof(*plan));
   hcj_frame_info &f = plan->info;
+  // HCJ_FLAG_LIBJPEG with a scaled decode: libjpeg reconstructs chroma at another block size there (not implemented)
+  if ((flags & HCJ_FLAG_LIBJPEG) && (flags & HCJ_FLAG_SCALE_MASK)) return HCJ_ERR_INVALID_ARG;
   if (!h.has_frame || !h.has_scan) return HCJ_ERR_NO_FRAME_OR_SCAN;  // decoder.ml:283-292
-  int max_h = 0, max_v = 0;                                           // decoder.ml:294-302
+  int max_h = 0, max_v = 0;                                          // decoder.ml:294-302
   for (int i = 0; i < h.number_of_components; i++) {
     max_h = std::max(max_h, h.components[i].horizontal_sampling_factor);
     max_v = std::max(max_v, h.components[i].vertical_sampling_factor);
@@ -363,6 +365,15 @@ int plan_image(const hcj_header &h, unsigned flags, ImagePlan *plan) {
     for (int i = 0; i < 3; i++) f.yuv_bytes += (size_t)f.actual_width[i] * f.actual_height[i];
     f.rgb_bytes = (size_t)f.width * f.height * 3;
   }
+  // HCJ_FLAG_LIBJPEG: jdsample.c up-samples every component by (h_max / h_c, v_max / v_c) when these are integral, so a
+  // 3-component frame of any such sampling (4:4:0, 4:1:1 too) has an RGB24 / YUV444 output
+  plan->up_integral = true;
+  for (int i = 0; i < ncomp; i++) {
+    plan->up_h[i] = max_h % f.hs[i] == 0 ? max_h / f.hs[i] : 0;
+    plan->up_v[i] = max_v % f.vs[i] == 0 ? max_v / f.vs[i] : 0;
+    plan->up_integral = plan->up_integral && plan->up_h[i] && plan->up_v[i];
+  }
+  if ((flags & HCJ_FLAG_LIBJPEG) && ncomp == 3 && plan->up_integral) f.rgb_bytes = (size_t)f.width * f.height * 3;
   return HCJ_OK;
 }
 

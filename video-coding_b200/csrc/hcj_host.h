@@ -28,6 +28,9 @@ struct ImagePlan {
   int dc_index[HCJ_MAX_COMPONENTS];       // index into header.huffman_tables
   int ac_index[HCJ_MAX_COMPONENTS];
   int blk_comp[HCJ_MAX_BPM], blk_bx[HCJ_MAX_BPM], blk_by[HCJ_MAX_BPM];
+  // libjpeg's up-sampling ratios (h_max / h_c, v_max / v_c), all components integral; HCJ_FLAG_LIBJPEG only
+  bool up_integral;
+  int up_h[HCJ_MAX_COMPONENTS], up_v[HCJ_MAX_COMPONENTS];
 };
 int plan_image(const hcj_header &h, unsigned flags, ImagePlan *plan);
 // HCJ_FLAG_SCALE_*: log2 of the scale denominator s (0 = full size, 1..3 = 1/2, 1/4, 1/8)

@@ -1640,6 +1640,35 @@ __device__ __forceinline__ void scaled_block_store(const uint4 *tile, int slot, 
   store_block_rows_k<K>(pix, dst, stride, x, y, stride, h_limit);
 }
 
+// HCJ_FLAG_LIBJPEG: one block of the staged tile reconstructed with libjpeg's islow IDCT and stored.  Flagged blocks and
+// 16-bit tables take the 64-bit column pass out of line (islow_wide).
+__device__ __noinline__ void islow_block_store_wide(const uint4 *tile, int slot, const int32_t *q, uint8_t *dst, int stride, int x,
+                                                    int y, int h_limit) {
+  uint32_t cw[32], pix[16];
+  for (int j = 0; j < 8; j++) {
+    const uint4 u = tile[slot * 8 + (j ^ (slot & 7))];
+    cw[4 * j] = u.x, cw[4 * j + 1] = u.y, cw[4 * j + 2] = u.z, cw[4 * j + 3] = u.w;
+  }
+  islow_wide(cw, q, pix);
+  store_block_rows(pix, dst, stride, x, y, stride, h_limit);
+}
+
+__device__ __forceinline__ void islow_block_store(const uint4 *tile, int slot, const int32_t *q, bool wide, uint8_t *dst, int stride,
+                                                  int x, int y, int h_limit) {
+  if (wide) {
+    islow_block_store_wide(tile, slot, q, dst, stride, x, y, h_limit);
+    return;
+  }
+  uint32_t cw[32], pix[16];
+#pragma unroll
+  for (int j = 0; j < 8; j++) {
+    const uint4 u = tile[slot * 8 + (j ^ (slot & 7))];
+    cw[4 * j] = u.x, cw[4 * j + 1] = u.y, cw[4 * j + 2] = u.z, cw[4 * j + 3] = u.w;
+  }
+  islow_fast(cw, q + 64, pix);
+  store_block_rows(pix, dst, stride, x, y, stride, h_limit);
+}
+
 // Persistent CTAs (HCJ_IDCT_CTAS_PER_SM per SM): each owns a contiguous range of the batch's tiles and keeps the coefficient
 // tile, the quant tables and the wide-block flags of tile i+1 in flight (cp.async) while tile i is being
 // transformed.  The thread -> block mapping depends only on (image geometry, tile width): it is computed
@@ -2071,7 +2100,8 @@ __device__ __forceinline__ void idct_tile_rgb_sub(const DecodeBatchDev &b, const
 // (idct_tile_rgb444 below); every other tile, and every tile of the FUSED = false instance, takes the planar path.
 // K: samples per block side in the output planes; K = 4, 2, 1 are the scaled decodes (HCJ_FLAG_SCALE_*, never fused),
 // which keep the tile plan, the staging and the thread -> block mapping and change only the transform and the store.
-template <bool FUSED, int K = 8>
+// ISLOW (K = 8, never fused) is the libjpeg reconstruction (HCJ_FLAG_LIBJPEG) in the same frame.
+template <bool FUSED, int K = 8, bool ISLOW = false>
 __global__ void __launch_bounds__(IDCT_MAX_THREADS, HCJ_IDCT_CTAS_PER_SM)
     k_idct_persistent(const __grid_constant__ DecodeBatchDev b, int mode) {
   extern __shared__ uint4 s_dyn[];
@@ -2148,13 +2178,14 @@ __global__ void __launch_bounds__(IDCT_MAX_THREADS, HCJ_IDCT_CTAS_PER_SM)
       idct_tile_rgb444(b, t, st, mp, tnow);
     } else if (FUSED && t.fused == 2u) {
       idct_tile_rgb_sub(b, t, st, mp, tnow);
-    } else if (K != 8 && (mp.misc & (1u << 10))) {
+    } else if ((K != 8 || ISLOW) && (mp.misc & (1u << 10))) {
       const int slot = (int)(mp.misc & 255u);
       const uint32_t fbit = (uint32_t)(t.blk0 & 127u) + slot;
       const bool wide = (mp.misc & (1u << 11)) || ((reinterpret_cast<const uint32_t *>(st.flags)[fbit >> 5] >> (fbit & 31u)) & 1u);
       const int x = (int)t.m0 * (int)((mp.misc >> 12) & 63u) + (int)(mp.xy & 0xffffu);
       const int y = (int)t.my * (int)((mp.misc >> 18) & 63u) + (int)(mp.xy >> 16);
-      scaled_block_store<K>(st.tile, slot, st.q + ((mp.misc >> 8) & 3u) * 128u, wide, mp.plane, mp.stride, x, y, mp.h_limit);
+      if (ISLOW) islow_block_store(st.tile, slot, st.q + ((mp.misc >> 8) & 3u) * 128u, wide, mp.plane, mp.stride, x, y, mp.h_limit);
+      else scaled_block_store<K>(st.tile, slot, st.q + ((mp.misc >> 8) & 3u) * 128u, wide, mp.plane, mp.stride, x, y, mp.h_limit);
     } else if (K == 8 && (mp.misc & (1u << 10))) {
       const int slot = (int)(mp.misc & 255u);
       uint32_t cw[32];
@@ -2192,7 +2223,8 @@ void launch_idct(const DecodeBatchDev &b, int mode, cudaStream_t s) {
   k_idct_plan<<<dim3((b.max_idct_tiles + 127) / 128, b.img_hi - b.img_lo), 128, 0, s>>>(b);
   const uint32_t total = b.tile_hi - b.tile_lo;
   const unsigned ctas = (unsigned)(total < (uint32_t)grid ? total : grid);
-  if (b.block_k == 4) k_idct_persistent<false, 4><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  if (b.islow) k_idct_persistent<false, 8, true><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
+  else if (b.block_k == 4) k_idct_persistent<false, 4><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
   else if (b.block_k == 2) k_idct_persistent<false, 2><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
   else if (b.block_k == 1) k_idct_persistent<false, 1><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
   else if (mode == 2 && (b.has_fused || b.has_fused_sub)) k_idct_persistent<true><<<ctas, IDCT_MAX_THREADS, IDCT_SMEM, s>>>(b, mode);
@@ -2574,6 +2606,126 @@ __global__ void __launch_bounds__(128) k_rgb444_fix(DecodeBatchDev b) {
   }
 }
 
+// ================================================================================================
+// K9 for HCJ_FLAG_LIBJPEG: libjpeg's up-sampling (jdsample.c, libjpeg_upsample in hcj_device.cuh) + the colour formula,
+// for the images that are not 4:4:4 (those take k_rgb: libjpeg's copy is Planar_444's).  One thread per 16 horizontally
+// adjacent pixels of a row.  The common layouts - luma at full size, both chroma components at ratio (2, 1) or (2, 2),
+// real chroma planes wider than 2 - take the fast path: 16 luma samples and, per chroma component, 8 samples with their
+// left and right neighbours from one row (h2v1) or from the near and the far row (h2v2), all requested before anything
+// is computed.  Only the group at the right end of the real chroma plane (EDGE) replicates its last sample inside the
+// group.  Everything else (4:4:0, 4:1:1, other layouts, planes of width <= 2) goes sample by sample.
+// ================================================================================================
+struct ChromaRow10 {
+  uint2 m;   // samples j0 .. j0 + 7
+  int l, r;  // samples j0 - 1 and j0 + 8, clamped to the real plane
+};
+__device__ __forceinline__ ChromaRow10 load_chroma_row10(const uint8_t *row, int j0, int rw) {
+  ChromaRow10 t;
+  t.m = __ldg(reinterpret_cast<const uint2 *>(row + j0));
+  t.l = __ldg(row + max(j0 - 1, 0));
+  t.r = __ldg(row + min(j0 + 8, rw - 1));
+  return t;
+}
+template <bool EDGE>
+__device__ __forceinline__ void unpack_chroma_row10(const ChromaRow10 &t, int j0, int rw, int (&a)[10]) {
+  a[0] = t.l;
+#pragma unroll
+  for (int k = 0; k < 8; k++) a[k + 1] = (int)(((k < 4 ? t.m.x : t.m.y) >> (8 * (k & 3))) & 0xffu);
+  if (EDGE)
+#pragma unroll
+    for (int k = 1; k < 8; k++)  // past the real plane: its last sample, libjpeg's right edge
+      if (j0 + k > rw - 1) a[k + 1] = a[k];
+  a[9] = t.r;
+}
+// h2v1_fancy_upsample (V2 = false: `near` only) or h2v2_fancy_upsample of 8 chroma samples -> 16, packed into w[4].
+template <bool V2, bool EDGE>
+__device__ __forceinline__ void fancy16(const ChromaRow10 &nr, const ChromaRow10 &fr, int j0, int rw, uint32_t (&w)[4]) {
+  int a[10];
+  unpack_chroma_row10<EDGE>(nr, j0, rw, a);
+  if (V2) {
+    int f[10];
+    unpack_chroma_row10<EDGE>(fr, j0, rw, f);
+#pragma unroll
+    for (int k = 0; k < 10; k++) a[k] = 3 * a[k] + f[k];  // column sums
+  }
+#pragma unroll
+  for (int k = 0; k < 8; k++) {
+    const int c3 = 3 * a[k + 1];
+    const uint32_t lo = V2 ? (uint32_t)(c3 + a[k] + 8) >> 4 : (uint32_t)(c3 + a[k] + 1) >> 2;
+    const uint32_t hi = V2 ? (uint32_t)(c3 + a[k + 2] + 7) >> 4 : (uint32_t)(c3 + a[k + 2] + 2) >> 2;
+    if (k & 1) w[k >> 1] |= (lo | hi << 8) << 16;
+    else w[k >> 1] = lo | hi << 8;
+  }
+}
+
+template <bool PLANAR>  // PLANAR: planar 4:4:4 Y, U, V (HCJ_OUT_YUV444) instead of RGB24
+__global__ void __launch_bounds__(128) k_rgb_libjpeg(DecodeBatchDev b) {
+  const HcjImageDesc &d = b.descs[blockIdx.z + b.img_lo];
+  if (!d.valid || !d.libjpeg) return;
+  const int x0 = (blockIdx.x * blockDim.x + threadIdx.x) * 16, y = blockIdx.y;
+  if (y >= d.height || x0 >= d.width) return;
+  const int n = min(16, d.width - x0);
+  const HcjCompGeom &gy = d.comp[0], &gu = d.comp[1], &gv = d.comp[2];
+  const uint8_t *py = b.planes + gy.plane_off, *pu = b.planes + gu.plane_off, *pv = b.planes + gv.plane_off;
+  const int hr = gu.up_h, vr = gu.up_v;
+  const int rw = (d.width + hr - 1) / hr, rh = (d.height + vr - 1) / vr;  // the real chroma plane
+  uint32_t wy[4], wu[4], wv[4];
+  if (gy.up_h == 1 && gy.up_v == 1 && hr == 2 && vr <= 2 && gv.up_h == 2 && gv.up_v == vr && rw > 2) {
+    const int j0 = x0 >> 1, i = y / vr;
+    const int fi = vr == 2 ? min(max(i + ((y & 1) ? 1 : -1), 0), rh - 1) : i;
+    load16(py + (size_t)y * gy.decoded_w + x0, wy);
+    const ChromaRow10 un = load_chroma_row10(pu + (size_t)i * gu.decoded_w, j0, rw), vn = load_chroma_row10(pv + (size_t)i * gv.decoded_w, j0, rw);
+    const ChromaRow10 uf = load_chroma_row10(pu + (size_t)fi * gu.decoded_w, j0, rw), vf = load_chroma_row10(pv + (size_t)fi * gv.decoded_w, j0, rw);
+    const bool edge = j0 + 8 > rw - 1;
+    if (vr == 2) {
+      if (edge) fancy16<true, true>(un, uf, j0, rw, wu), fancy16<true, true>(vn, vf, j0, rw, wv);
+      else fancy16<true, false>(un, uf, j0, rw, wu), fancy16<true, false>(vn, vf, j0, rw, wv);
+    } else {
+      if (edge) fancy16<false, true>(un, uf, j0, rw, wu), fancy16<false, true>(vn, vf, j0, rw, wv);
+      else fancy16<false, false>(un, uf, j0, rw, wu), fancy16<false, false>(vn, vf, j0, rw, wv);
+    }
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; k++) wy[k] = wu[k] = wv[k] = 0u;
+#pragma unroll
+    for (int i = 0; i < 16; i++) {
+      if (i >= n) break;
+      const int x = x0 + i, sh = 8 * (i & 3);
+      const HcjCompGeom *g[3] = {&gy, &gu, &gv};
+      const uint8_t *p[3] = {py, pu, pv};
+      uint32_t v[3];
+#pragma unroll
+      for (int c = 0; c < 3; c++) {
+        const int h = g[c]->up_h, vv = g[c]->up_v;
+        v[c] = (uint32_t)libjpeg_upsample(p[c], g[c]->decoded_w, (d.width + h - 1) / h, (d.height + vv - 1) / vv, h, vv, x, y);
+      }
+      wy[i >> 2] |= v[0] << sh;
+      wu[i >> 2] |= v[1] << sh;
+      wv[i >> 2] |= v[2] << sh;
+    }
+  }
+  if (PLANAR) {
+    const size_t plane = (size_t)d.width * d.height;
+    uint8_t *oy = b.out + d.out_off + (size_t)y * d.width + x0;
+    store_any<4>(oy, wy, n);
+    store_any<4>(oy + plane, wu, n);
+    store_any<4>(oy + 2 * plane, wv, n);
+    return;
+  }
+  uint32_t o[12];
+#pragma unroll
+  for (int k = 0; k < 4; k++) {  // 4 pixels -> 12 bytes = 3 words
+    uint32_t px[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++)
+      px[i] = ycc_to_rgb((wy[k] >> (8 * i)) & 0xff, (wu[k] >> (8 * i)) & 0xff, (wv[k] >> (8 * i)) & 0xff);
+    o[3 * k + 0] = px[0] | (px[1] << 24);
+    o[3 * k + 1] = (px[1] >> 8) | (px[2] << 16);
+    o[3 * k + 2] = (px[2] >> 16) | (px[3] << 8);
+  }
+  store_any<12>(b.out + d.out_off + ((size_t)y * d.width + x0) * 3, o, 3 * n);
+}
+
 void launch_rgb(const DecodeBatchDev &b, bool planar444, cudaStream_t s) {
   if (b.img_hi <= b.img_lo || b.max_rgb_rows == 0) return;
   if (!planar444 && b.has_fused && b.max_blocks)
@@ -2593,6 +2745,10 @@ void launch_rgb(const DecodeBatchDev &b, bool planar444, cudaStream_t s) {
       if (b.has_subsampled & 1) k_rgb_sub_pairs<<<dim3(grid.x, (b.max_rgb_rows + 1) / 2, grid.z), block, 0, s>>>(b);
       if (b.has_subsampled & 2) k_rgb<false, true><<<grid, block, 0, s>>>(b);
     }
+  }
+  if (b.has_libjpeg) {
+    if (planar444) k_rgb_libjpeg<true><<<grid, block, 0, s>>>(b);
+    else k_rgb_libjpeg<false><<<grid, block, 0, s>>>(b);
   }
 }
 
@@ -2774,6 +2930,7 @@ int configure_device(int *sm_count) {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(k_idct_persistent<false, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IDCT_SMEM);
   if (sm_count) *sm_count = sms;
   return (int)e;
 }

@@ -72,6 +72,9 @@ struct DecodeBatchDev {
   uint32_t img_lo, img_hi;        // images [img_lo, img_hi)
   uint32_t lr_lo, lr_hi;          // entries of list_restart
   uint32_t ls_lo, ls_hi;          // entries of list_spec
+  // HCJ_FLAG_LIBJPEG (kept behind the fields above so that their offsets, and the other kernels' code, stay as they were)
+  int islow;                      // k_idct_persistent reconstructs with libjpeg's islow IDCT
+  int has_libjpeg;                // the batch holds images that k_rgb_libjpeg up-samples (HcjImageDesc::libjpeg)
 };
 
 // Once per context, with its device current: shared-memory opt-ins of the kernels (a per-device attribute) and the

@@ -28,6 +28,9 @@ FLAG_SCALE_1_2 = 0x10
 FLAG_SCALE_1_4 = 0x20
 FLAG_SCALE_1_8 = 0x30
 FLAG_SCALE_MASK = 0x30
+# libjpeg-turbo's default reconstruction (stated extension, include/hcjpeg.h): islow IDCT and fancy chroma up-sampling, so
+# RGB24 equals Pillow / OpenCV.  Not combinable with FLAG_SCALE_*.
+FLAG_LIBJPEG = 0x40
 ENC_SRC_DEVICE = 1  # hcj_encode_rgb_batch: the frames are device pointers on the context's device
 
 MAX_COMPONENTS = 4
