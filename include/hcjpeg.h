@@ -273,6 +273,14 @@ int hcj_encode_batch(hcj_ctx *ctx, const uint8_t *const *yuv, int n, int width, 
 int hcj_encode_batch_multi(hcj_ctx *const *ctx, int nctx, const uint8_t *const *yuv, int n, int width, int height, int chroma,
                            int quality, int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
                            int *status);
+/* hcj_encode_batch / hcj_encode_batch_multi with encode flags: HCJ_ENC_OPTIMIZE_HUFFMAN, or 0 (the same files as
+ * hcj_encode_batch); any other bit is HCJ_ERR_INVALID_ARG before any work, with nothing written. */
+int hcj_encode_batch_ex(hcj_ctx *ctx, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
+                        int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
+                        int *status);
+int hcj_encode_batch_multi_ex(hcj_ctx *const *ctx, int nctx, const uint8_t *const *yuv, int n, int width, int height, int chroma,
+                              int quality, int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity,
+                              size_t *out_len, int *status);
 /* The same for RGB24 frames (extension; the model's encoder takes planar frames only): rgb[i] is width*height*3 bytes,
  * R, G, B interleaved, rows top to bottom, no padding - the layout HCJ_OUT_RGB24 decodes to.  On the device, every frame
  * is taken to the planar frame of `chroma` that hcj_encode_batch would be given, in two steps:
@@ -287,9 +295,25 @@ int hcj_encode_batch_multi(hcj_ctx *const *ctx, int nctx, const uint8_t *const *
  * That frame is then encoded exactly as hcj_encode_batch encodes it: the files are byte-identical, statuses (for
  * example HCJ_ERR_PLANE_BOUNDS), out_len, HCJ_ERR_BUFFER_TOO_SMALL, hcj_encode_bound and hcj_encode_last_device_ms
  * (which includes the conversion) behave the same.  Without flags the frames are in host memory and go up chunk by
- * chunk like planar frames (3 bytes a pixel instead of 1.5 for 4:2:0).  flags: HCJ_ENC_SRC_DEVICE, or 0; other bits
- * are HCJ_ERR_INVALID_ARG. */
+ * chunk like planar frames (3 bytes a pixel instead of 1.5 for 4:2:0).  flags: HCJ_ENC_SRC_DEVICE and / or
+ * HCJ_ENC_OPTIMIZE_HUFFMAN, or 0; other bits are HCJ_ERR_INVALID_ARG. */
 #define HCJ_ENC_SRC_DEVICE 1u /* rgb[i] are device pointers on the context's device */
+/* Extension (the model always writes the four Annex K tables): every frame gets its own optimal Huffman tables, as
+ * Pillow optimize=True, OpenCV IMWRITE_JPEG_OPTIMIZE and cjpeg -optimize make them.  Frame i is encoded as follows:
+ *   1. the quantised coefficients, MCU order, restart intervals and statuses are those of the default encode;
+ *   2. per table (dc 0 / ac 0: Y blocks; dc 1 / ac 1: Cb and Cr blocks; 400 has table 0 only), the symbols the default
+ *      encode of frame i codes are counted: the DC size of every DC difference, one ZRL per 16 zeros before a non-zero
+ *      AC coefficient, (run << 4) | size per non-zero AC coefficient, an EOB when coefficient 63 is zero;
+ *   3. each table is libjpeg's jpeg_gen_optimal_table (jchuff.c, T.81 Annex K.2) of those counts with the reserved
+ *      all-ones code; code sizes above 32 before the length limit are no error; HUFFVAL is ordered by the code size
+ *      before the limit, then by symbol;
+ *   4. the file is the default file's header with each DHT segment (same order, same class / id) carrying frame i's
+ *      table, then the scan coded with those tables, then EOI.
+ * Decoders give exactly the pixels of the default file.  Headers are never longer than the default one and a block never
+ * needs more bits than with the Annex K tables, so hcj_encode_bound holds; statuses, out_len with
+ * HCJ_ERR_BUFFER_TOO_SMALL and hcj_encode_last_device_ms (which includes the two kernels this adds) behave as without
+ * the flag.  Taken by hcj_encode_batch_ex, hcj_encode_batch_multi_ex and hcj_encode_rgb_batch. */
+#define HCJ_ENC_OPTIMIZE_HUFFMAN 0x100u
 /* With HCJ_ENC_SRC_DEVICE nothing is uploaded: the conversion reads the caller's buffers, on the context's stream (the
  * one passed to hcj_ctx_create), so work the caller enqueued on that stream before the call is ordered before the
  * reads; work on other streams must be synchronised by the caller.  Every pointer is checked before any work is
@@ -302,7 +326,7 @@ int hcj_encode_rgb_batch(hcj_ctx *ctx, const uint8_t *const *rgb, int n, int wid
  * (width*height bytes of Y, then Cb and Cr; Y only for 400).  HCJ_ERR_BUFFER_TOO_SMALL if dst_capacity is less. */
 int hcj_rgb_to_yuv(hcj_ctx *ctx, const uint8_t *rgb, int width, int height, int chroma, uint8_t *dst, size_t dst_capacity);
 size_t hcj_encode_bound(int width, int height, int chroma); /* worst-case bytes of one encoded frame */
-int hcj_encode_count_kernels(void); /* kernels one hcj_encode_batch launches */
+int hcj_encode_count_kernels(void); /* kernels one hcj_encode_batch launches (HCJ_ENC_OPTIMIZE_HUFFMAN adds two per chunk) */
 /* Encoder.write_headers (encoder.ml:371-418).  Host only. */
 int hcj_write_headers(int width, int height, int chroma, int quality, int restart_interval, uint8_t *out,
                       size_t capacity, size_t *len);

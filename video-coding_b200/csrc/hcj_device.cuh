@@ -1329,6 +1329,256 @@ HCJ_HD bool encode_block_fields_sparse(uint64_t nz, Coef coef, int32_t dcdiff, c
   return ok;
 }
 
+// ------------------------------------------------------------------------------------------------
+// Optimal Huffman tables (HCJ_ENC_OPTIMIZE_HUFFMAN, DESIGN.md 5)
+// ------------------------------------------------------------------------------------------------
+// The symbols encode_block_fields_sparse codes, in the same order and by the same control flow: visit(is_ac, symbol)
+// for the DC size, every ZRL, every (run << 4) | size and the EOB.  A coefficient of size 16 or more has no symbol:
+// it is not visited and the result is false (encode_block_fields_sparse reports it as a missing code).
+template <class Coef, class Visit>
+HCJ_HD bool block_symbols_sparse(uint64_t nz, Coef coef, int32_t dcdiff, Visit &visit) {
+  bool ok = true;
+  uint32_t size = coef_size(dcdiff);
+  if (size < 16u) visit(false, size);
+  else ok = false;
+  int prev = 0;
+  for (uint64_t m = nz & ~1ull; m; m &= m - 1ull) {
+    const int k = lowest_bit(m);
+    uint32_t run = (uint32_t)(k - prev - 1);
+    prev = k;
+    for (; run >= 16u; run -= 16u) visit(true, 0xf0u);
+    size = coef_size(coef(k));
+    if (size < 16u) visit(true, (run << 4) | size);
+    else ok = false;
+  }
+  if (prev != 63) visit(true, 0x00u);
+  return ok;
+}
+
+// The symbols the four Annex K tables code (12 DC sizes; 160 (run, size) pairs with size 1..10, EOB, ZRL): a frame that
+// needs any other symbol gets the status the default tables give it.
+HCJ_HD bool annex_k_symbol(bool is_ac, uint32_t sym) {
+  if (!is_ac) return sym <= 11u;
+  const uint32_t size = sym & 15u;
+  return sym == 0x00u || sym == 0xf0u || (size >= 1u && size <= 10u);
+}
+
+// Code sizes above 16 before the limit need this many entries: the counts of a frame are below 2^32, and a code of
+// length L needs a total of at least Fibonacci(L + 2).
+constexpr int HCJ_K2_MAX_CLEN = 64;
+
+// libjpeg's jpeg_gen_optimal_table (jchuff.c; T.81 Annex K.2) for freq[0..255] and the reserved freq[256] = 1: the
+// specification the warp procedure (k2_optimal_table) is checked against.  Unlike libjpeg, code sizes above 32 before
+// the limit are not an error.  HUFFVAL is ordered by the code size before the limit, then by symbol.  Returns the
+// number of symbols.
+HCJ_HD int gen_optimal_table(const uint32_t freq_in[257], uint8_t bits_out[16], uint8_t huffval[256]) {
+  uint32_t freq[257];
+  int codesize[257], others[257];
+  for (int i = 0; i < 257; i++) {
+    freq[i] = i < 256 ? freq_in[i] : 1u;
+    codesize[i] = 0;
+    others[i] = -1;
+  }
+  for (;;) {
+    int c1 = -1, c2 = -1;
+    uint64_t v = ~0ull;
+    for (int i = 0; i <= 256; i++)
+      if (freq[i] && freq[i] <= v) v = freq[i], c1 = i;
+    v = ~0ull;
+    for (int i = 0; i <= 256; i++)
+      if (freq[i] && freq[i] <= v && i != c1) v = freq[i], c2 = i;
+    if (c2 < 0) break;
+    freq[c1] += freq[c2];
+    freq[c2] = 0;
+    codesize[c1]++;
+    while (others[c1] >= 0) {
+      c1 = others[c1];
+      codesize[c1]++;
+    }
+    others[c1] = c2;
+    codesize[c2]++;
+    while (others[c2] >= 0) {
+      c2 = others[c2];
+      codesize[c2]++;
+    }
+  }
+  int bits[HCJ_K2_MAX_CLEN] = {0};
+  for (int i = 0; i <= 256; i++)
+    if (codesize[i]) bits[codesize[i]]++;
+  int i = HCJ_K2_MAX_CLEN - 1;
+  for (; i > 16; i--)
+    while (bits[i] > 0) {
+      int j = i - 2;
+      while (bits[j] == 0) j--;
+      bits[i] -= 2;
+      bits[i - 1]++;
+      bits[j + 1] += 2;
+      bits[j]--;
+    }
+  while (i > 0 && bits[i] == 0) i--;
+  if (i > 0) bits[i]--;
+  for (int l = 0; l < 16; l++) bits_out[l] = (uint8_t)bits[l + 1];
+  int p = 0;
+  for (int l = 1; l < HCJ_K2_MAX_CLEN; l++)
+    for (int j = 0; j <= 255; j++)
+      if (codesize[j] == l) huffval[p++] = (uint8_t)j;
+  return p;
+}
+
+// The lanes that run k2_optimal_table together: the 32 lanes of a warp in k_huff_tables, one lane in the CPU emulation
+// (which then does every lane's share itself).
+struct K2Lanes {
+  int lane, size;
+  HCJ_HD void sync() const {
+#if defined(__CUDA_ARCH__)
+    __syncwarp();
+#endif
+  }
+  HCJ_HD uint64_t min(uint64_t v) const {
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+      const uint64_t o = __shfl_xor_sync(0xffffffffu, v, s);
+      v = o < v ? o : v;
+    }
+#endif
+    return v;
+  }
+  // number of lanes below this one with p set; *total: all lanes with p set
+  HCJ_HD uint32_t count_below(bool p, uint32_t *total) const {
+#if defined(__CUDA_ARCH__)
+    const uint32_t b = __ballot_sync(0xffffffffu, p);
+    *total = (uint32_t)__popc(b);
+    return (uint32_t)__popc(b & ((1u << lane) - 1u));
+#else
+    *total = p ? 1u : 0u;
+    return 0u;
+#endif
+  }
+};
+
+struct K2Scratch {  // one table's working set (shared memory in k_huff_tables)
+  uint32_t freq[257];
+  uint16_t sym[257];
+  int16_t others[257];
+  uint8_t codesize[257];
+  int32_t bits[HCJ_K2_MAX_CLEN];
+  uint32_t start[HCJ_K2_MAX_CLEN];
+  int n;
+};
+
+// gen_optimal_table by a group of lanes.  The non-zero symbols (and the reserved one, last) are compacted in symbol
+// order; each merge step finds c1 and c2 with two arg-min reductions over the key (frequency, larger index first);
+// lane 0 walks the `others` chains; HUFFVAL is a counting sort over (code size before the limit, symbol).  Same
+// bits_out / huffval / result as gen_optimal_table.
+HCJ_HD int k2_optimal_table(const K2Lanes &w, const uint32_t *freq_in /* [256] */, K2Scratch &s, uint8_t bits_out[16],
+                            uint8_t huffval[256]) {
+  uint32_t base = 0;
+  for (int i0 = 0; i0 < 257; i0 += w.size) {  // compaction (every lane runs the same number of rounds)
+    const int i = i0 + w.lane;
+    const uint32_t f = i < 256 ? freq_in[i] : i == 256 ? 1u : 0u;
+    uint32_t total;
+    const uint32_t at = base + w.count_below(f != 0u, &total);
+    if (f) {
+      s.freq[at] = f;
+      s.sym[at] = (uint16_t)i;
+      s.others[at] = -1;
+      s.codesize[at] = 0;
+    }
+    base += total;
+  }
+  const int n = (int)base;
+  for (int i = w.lane; i < HCJ_K2_MAX_CLEN; i += w.size) s.bits[i] = 0, s.start[i] = 0;
+  w.sync();
+  for (;;) {
+    // key: frequency above, the complement of the index below: the smallest key is the smallest frequency, and among
+    // equal frequencies the largest index (libjpeg's `<=` scan)
+    uint64_t k1 = ~0ull;
+    for (int i = w.lane; i < n; i += w.size)
+      if (s.freq[i]) {
+        const uint64_t k = ((uint64_t)s.freq[i] << 32) | (uint32_t)(0xffffu - i);
+        k1 = k < k1 ? k : k1;
+      }
+    k1 = w.min(k1);
+    const int c1 = 0xffff - (int)(uint32_t)(k1 & 0xffffffffu);
+    uint64_t k2 = ~0ull;
+    for (int i = w.lane; i < n; i += w.size)
+      if (s.freq[i] && i != c1) {
+        const uint64_t k = ((uint64_t)s.freq[i] << 32) | (uint32_t)(0xffffu - i);
+        k2 = k < k2 ? k : k2;
+      }
+    k2 = w.min(k2);
+    if (k2 == ~0ull) break;
+    const int c2 = 0xffff - (int)(uint32_t)(k2 & 0xffffffffu);
+    if (w.lane == 0) {
+      s.freq[c1] += s.freq[c2];
+      s.freq[c2] = 0;
+      int a = c1, b = c2;
+      s.codesize[a]++;
+      while (s.others[a] >= 0) {
+        a = s.others[a];
+        s.codesize[a]++;
+      }
+      s.others[a] = (int16_t)b;
+      s.codesize[b]++;
+      while (s.others[b] >= 0) {
+        b = s.others[b];
+        s.codesize[b]++;
+      }
+    }
+    w.sync();
+  }
+  if (w.lane == 0) {
+    // bits[] before the limit; start[l]: HUFFVAL position of the first symbol of code size l (the reserved symbol, the
+    // last one, takes no position)
+    for (int i = 0; i < n; i++)
+      if (s.codesize[i]) {
+        s.bits[s.codesize[i]]++;
+        if (i < n - 1) s.start[s.codesize[i]]++;
+      }
+    uint32_t acc = 0;
+    for (int l = 0; l < HCJ_K2_MAX_CLEN; l++) {
+      const uint32_t c = s.start[l];
+      s.start[l] = acc;
+      acc += c;
+    }
+    int i = HCJ_K2_MAX_CLEN - 1;
+    for (; i > 16; i--)
+      while (s.bits[i] > 0) {
+        int j = i - 2;
+        while (s.bits[j] == 0) j--;
+        s.bits[i] -= 2;
+        s.bits[i - 1]++;
+        s.bits[j + 1] += 2;
+        s.bits[j]--;
+      }
+    while (i > 0 && s.bits[i] == 0) i--;
+    if (i > 0) s.bits[i]--;
+    for (int l = 0; l < 16; l++) bits_out[l] = (uint8_t)s.bits[l + 1];
+  }
+  w.sync();
+  // symbols of equal code size keep their (symbol) order: rank = the ones of that size before it
+  for (int i = w.lane; i < n - 1; i += w.size) {
+    const uint8_t cs = s.codesize[i];
+    uint32_t r = s.start[cs];
+    for (int j = 0; j < i; j++) r += s.codesize[j] == cs;
+    huffval[r] = (uint8_t)s.sym[i];
+  }
+  w.sync();
+  return n - 1;
+}
+
+// Canonical codes of (bits, huffval) (T.81 Annex C) as (code << 8) | length: dc[symbol & 15] or ac[symbol], the format
+// the encode kernels read.  Entries of symbols the table does not hold are left alone.
+HCJ_HD void canonical_codes(const uint8_t bits[16], const uint8_t *huffval, bool dc, uint32_t *codes) {
+  uint32_t code = 0;
+  int p = 0;
+  for (int l = 0; l < 16; l++) {
+    for (int i = 0; i < bits[l]; i++, p++) codes[dc ? (huffval[p] & 15) : huffval[p]] = ((code + i) << 8) | (uint32_t)(l + 1);
+    code = (code + bits[l]) << 1;
+  }
+}
+
 // coefficient k of a block held as 32 words of two int16 each (the layout of the coefficient buffer)
 HCJ_HD int32_t packed_coef(const uint32_t *qw, int k) {
   const uint32_t w = qw[k >> 1];

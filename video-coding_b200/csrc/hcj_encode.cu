@@ -5,6 +5,10 @@
 //                            into its own 512-bit slot, and their length in bits (the field loop runs once per block:
 //                            the block staged in shared memory, one iteration per non-zero coefficient,
 //                            encode_block_fields_sparse)
+//   k_symbol_counts  HCJ_ENC_OPTIMIZE_HUFFMAN only, before k_block_bits: per frame and table, the counts of the symbols the
+//                    default encode codes (block_symbols_sparse)
+//   k_huff_tables    HCJ_ENC_OPTIMIZE_HUFFMAN only: per frame, libjpeg's K.2 tables (one warp per table) as the codes
+//                    k_block_bits / k_pack read, and the frame's header with those DHT segments, which k_seg_scan copies
 //   k_scan_bits    per frame: exclusive prefix sum of block bit lengths (one CTA walks the frame)
 //   k_place        E8,E9     per block: the finished bit string shifted to its bit offset (big-endian 32-bit words,
 //                            atomicOr only on the two boundary words), 1-fill at the end of every segment
@@ -144,9 +148,10 @@ struct EncTablesSmem {
   uint32_t ac[2][256];
 };
 
-__device__ __forceinline__ void load_enc_tables(EncTablesSmem &t, const EncodeBatchDev &e) {
-  for (int i = threadIdx.x; i < 32; i += blockDim.x) t.dc[i >> 4][i & 15] = e.dc_codes[i];
-  for (int i = threadIdx.x; i < 512; i += blockDim.x) t.ac[i >> 8][i & 255] = e.ac_codes[i];
+__device__ __forceinline__ void load_enc_tables(EncTablesSmem &t, const EncodeBatchDev &e, uint32_t frame) {
+  const uint32_t *dc = e.dc_codes + (uint64_t)frame * e.tab_stride, *ac = e.ac_codes + (uint64_t)frame * e.tab_stride;
+  for (int i = threadIdx.x; i < 32; i += blockDim.x) t.dc[i >> 4][i & 15] = dc[i];
+  for (int i = threadIdx.x; i < 512; i += blockDim.x) t.ac[i >> 8][i & 255] = ac[i];
 }
 
 // The 128 blocks of a CTA are one contiguous 16 KiB run of the coefficient buffer: the CTA copies it into shared memory
@@ -208,7 +213,7 @@ struct LocalPacker {
 // ---- K7a -----------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(128) k_block_bits(EncodeBatchDev e, int *status) {
   __shared__ EncTablesSmem t;
-  load_enc_tables(t, e);
+  load_enc_tables(t, e, blockIdx.y);
   __syncthreads();
   const uint32_t blk = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t frame = blockIdx.y;
@@ -229,6 +234,96 @@ __global__ void __launch_bounds__(128) k_block_bits(EncodeBatchDev e, int *statu
   if (!ok) atomicCAS(status + frame, 0, HCJ_ERR_ENCODER_PARAMS);
   e.blk_bits[(uint64_t)frame * (e.nblocks + 1) + blk] = pk.bits;
   if (pk.bits > (uint32_t)HCJ_ENC_SLOT_WORDS * 32u) *e.long_blocks = 1u;  // (every writer stores the same value)
+}
+
+// ---- K7o: symbol counts of every frame (HCJ_ENC_OPTIMIZE_HUFFMAN) ----------------------------------
+// k_block_bits's grid and staging, block_symbols_sparse instead of the field loop.  counts[frame][4][256]: tables dc 0,
+// dc 1, ac 0, ac 1 (Y blocks take table 0, Cb and Cr table 1), zeroed by the chunk's memsets.  Each CTA counts into
+// shared memory and adds its non-zero bins to the frame's counts.  The DC size and the EOB, which almost every lane of
+// a warp visits at the same point, are summed over the lanes that share the bin before the shared atomic.
+__global__ void __launch_bounds__(128) k_symbol_counts(EncodeBatchDev e, uint32_t *counts, int *status) {
+  __shared__ uint32_t s_hist[4 * 256];
+  __shared__ __align__(16) uint32_t s_rows[128 * ENC_ROW_WORDS];
+  for (int i = threadIdx.x; i < 4 * 256; i += blockDim.x) s_hist[i] = 0;
+  const uint32_t blk = blockIdx.x * blockDim.x + threadIdx.x;
+  const uint32_t frame = blockIdx.y;
+  stage_cta_blocks(e.quant + (uint64_t)frame * e.nblocks * 64, blockIdx.x * blockDim.x, e.nblocks, s_rows);  // (barrier)
+  if (blk < e.nblocks) {
+    const uint32_t *row = s_rows + threadIdx.x * ENC_ROW_WORDS;
+    const uint64_t nz = row_nonzero_map(row);
+    const int16_t *row16 = reinterpret_cast<const int16_t *>(row);
+    int64_t pb = dc_pred_block(e, blk);
+    int32_t pred = pb < 0 ? 0 : (int32_t)e.quant[((uint64_t)frame * e.nblocks + pb) * 64];
+    const int tsel = e.blk_comp[blk % e.bpm] ? 1 : 0;
+    bool legal = true;
+    auto visit = [&](bool is_ac, uint32_t sym) {
+      legal &= annex_k_symbol(is_ac, sym);
+      const uint32_t bin = ((is_ac ? 2u : 0u) + tsel) * 256u + sym;
+      if (!is_ac || sym == 0x00u) {
+        const uint32_t peers = __match_any_sync(__activemask(), bin);
+        if ((threadIdx.x & 31u) == (uint32_t)(__ffs(peers) - 1)) atomicAdd(s_hist + bin, (uint32_t)__popc(peers));
+      } else {
+        atomicAdd(s_hist + bin, 1u);
+      }
+    };
+    const bool ok = block_symbols_sparse(nz, [row16](int k) { return (int32_t)row16[k]; }, (int32_t)row16[0] - pred, visit);
+    // a symbol the default tables lack: the status the default encode reports (k_block_bits)
+    if (!ok || !legal) atomicCAS(status + frame, 0, HCJ_ERR_ENCODER_PARAMS);
+  }
+  __syncthreads();
+  uint32_t *dst = counts + (uint64_t)frame * 4 * 256;
+  for (int i = threadIdx.x; i < 4 * 256; i += blockDim.x) {
+    const uint32_t v = s_hist[i];
+    if (v) atomicAdd(dst + i, v);
+  }
+}
+
+// ---- K7t: the optimal tables and the header of every frame (HCJ_ENC_OPTIMIZE_HUFFMAN) -------------------
+// One CTA per frame, one warp per table (dc 0, dc 1, ac 0, ac 1; warps 1 and 3 idle for 400).  Each warp runs K.2
+// (k2_optimal_table) on its counts and writes the canonical codes into the frame's slot of `tables` ([tab_stride]
+// words: dc[2][16], then ac[2][256], the layout of the shared default tables).  Then the CTA writes the frame's header:
+// the shared header's bytes before its first DHT segment, the four (two) DHT segments with this frame's tables in the
+// same order and with the same class / id bytes, the shared header's bytes after its last DHT segment.
+__global__ void __launch_bounds__(128) k_huff_tables(EncodeBatchDev e, const uint32_t *counts, uint32_t *tables, uint8_t *headers,
+                                                     uint32_t *header_len, uint32_t dht_off, uint32_t dht_end) {
+  __shared__ K2Scratch s_k2[4];
+  __shared__ uint8_t s_bits[4][16];
+  __shared__ uint8_t s_val[4][256];
+  __shared__ int s_nv[4];
+  const uint32_t frame = blockIdx.x;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int ntab = e.ncomp == 1 ? 1 : 2, cls = warp >> 1, t = warp & 1;
+  const bool active = t < ntab;
+  if (active) {
+    const K2Lanes w{lane, 32};
+    const int nv = k2_optimal_table(w, counts + ((uint64_t)frame * 4 + warp) * 256, s_k2[warp], s_bits[warp], s_val[warp]);
+    uint32_t *tab = tables + (uint64_t)frame * e.tab_stride;
+    uint32_t *codes = cls ? tab + 32 + t * 256 : tab + t * 16;
+    for (int i = lane; i < (cls ? 256 : 16); i += 32) codes[i] = 0u;
+    __syncwarp();
+    if (lane == 0) {
+      canonical_codes(s_bits[warp], s_val[warp], cls == 0, codes);
+      s_nv[warp] = nv;
+    }
+  }
+  __syncthreads();
+  uint8_t *h = headers + (uint64_t)frame * e.frame_header_stride;
+  uint32_t seg_off[4], pos = dht_off;
+  for (int k = 0; k < 4; k++) {
+    seg_off[k] = pos;
+    if ((k & 1) < ntab) pos += 21u + (uint32_t)s_nv[k];  // FF C4, length, Tc Th, 16 counts, values (markers.ml:222-231)
+  }
+  const uint32_t suffix = e.header_len - dht_end;
+  for (uint32_t i = threadIdx.x; i < dht_off; i += blockDim.x) h[i] = e.header[i];
+  for (uint32_t i = threadIdx.x; i < suffix; i += blockDim.x) h[pos + i] = e.header[dht_end + i];
+  if (active) {
+    uint8_t *d = h + seg_off[warp];
+    const int nv = s_nv[warp], len = 19 + nv;
+    for (int i = lane; i < 21 + nv; i += 32)
+      d[i] = i == 0 ? 0xffu : i == 1 ? 0xc4u : i == 2 ? (uint8_t)(len >> 8) : i == 3 ? (uint8_t)len : i == 4 ? (uint8_t)((cls << 4) | t)
+             : i < 21 ? s_bits[warp][i - 5] : s_val[warp][i - 21];
+  }
+  if (threadIdx.x == 0) header_len[frame] = pos + suffix;
 }
 
 // ---- K7b: in-place exclusive scan of blk_bits per frame; entry [nblocks] receives the total ---------
@@ -364,7 +459,7 @@ __global__ void __launch_bounds__(128) k_pack(EncodeBatchDev e) {
   const bool mine = blk < e.nblocks && P[blk + 1] - P[blk] > (uint32_t)HCJ_ENC_SLOT_WORDS * 32u;
   if (!__syncthreads_or(mine)) return;  // CTA-uniform: almost every CTA leaves here
   __shared__ EncTablesSmem t;
-  load_enc_tables(t, e);
+  load_enc_tables(t, e, blockIdx.y);
   __syncthreads();
   __shared__ __align__(16) uint32_t s_rows[128 * ENC_ROW_WORDS];
   stage_cta_blocks(e.quant + (uint64_t)frame * e.nblocks * 64, blockIdx.x * blockDim.x, e.nblocks, s_rows);
@@ -443,9 +538,11 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_seg_scan(EncodeBatchDev e) {
   const uint32_t nunits = e.nseg * e.seg_chunks;
   uint32_t *sb = e.seg_bytes + (uint64_t)frame * (nunits + 1);
   uint8_t *out = e.out + (uint64_t)frame * e.out_stride;
-  for (uint32_t i = threadIdx.x; i < e.header_len; i += SCAN_THREADS) out[i] = e.header[i];
+  const uint8_t *header = e.frame_header ? e.frame_header + frame * e.frame_header_stride : e.header;
+  const uint32_t header_len = e.frame_header ? e.frame_header_len[frame] : e.header_len;
+  for (uint32_t i = threadIdx.x; i < header_len; i += SCAN_THREADS) out[i] = header[i];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t carry = e.header_len;
+  uint32_t carry = header_len;
   for (uint32_t base = 0; base < nunits; base += SCAN_THREADS) {
     uint32_t i = base + threadIdx.x;
     const bool rst = i < nunits && (i + 1) % e.seg_chunks == 0 && (i + 1) / e.seg_chunks < e.nseg;
@@ -703,7 +800,9 @@ void launch_encode(const EncodeBatchDev &e, cudaStream_t s) {
   k_fdct_quant<<<gb, 128, 0, s>>>(e);
 }
 
-int encode_kernel_count() { return 8; }  // k_fdct_quant, k_block_bits, k_scan_bits, k_gather_totals, k_place, k_seg_count, k_seg_scan, k_stuff (+ k_pack for chunks with long blocks)
+// k_fdct_quant, k_block_bits, k_scan_bits, k_gather_totals, k_place, k_seg_count, k_seg_scan, k_stuff (+ k_pack for chunks with
+// long blocks; + k_symbol_counts and k_huff_tables with HCJ_ENC_OPTIMIZE_HUFFMAN)
+int encode_kernel_count() { return 8; }
 
 // Gathers the per-frame totals of the bit scan into a dense array for one small D2H copy.
 __global__ void k_gather_totals(EncodeBatchDev e, uint32_t *totals) {
@@ -716,6 +815,20 @@ static void launch_bit_lengths(const EncodeBatchDev &e, int *d_status, uint32_t 
   k_block_bits<<<gb, 128, 0, s>>>(e, d_status);
   k_scan_bits<<<e.n, SCAN_THREADS, 0, s>>>(e);
   k_gather_totals<<<(e.n + 127) / 128, 128, 0, s>>>(e, d_totals);
+}
+
+// HCJ_ENC_OPTIMIZE_HUFFMAN: per-frame symbol counts, tables and headers, between k_fdct_quant and k_block_bits
+struct HuffOpt {
+  uint32_t *counts;      // [n][4][256], zeroed before every chunk
+  uint32_t *tables;      // [n][e.tab_stride]
+  uint8_t *headers;      // [n][e.frame_header_stride]
+  uint32_t *header_len;  // [n]
+  uint32_t dht_off, dht_end;  // the DHT segments of the shared header: bytes [dht_off, dht_end)
+};
+static void launch_huff_opt(const EncodeBatchDev &e, const HuffOpt &o, int *d_status, cudaStream_t s) {
+  dim3 gb((e.nblocks + 127) / 128, e.n);
+  k_symbol_counts<<<gb, 128, 0, s>>>(e, o.counts, d_status);
+  k_huff_tables<<<e.n, 128, 0, s>>>(e, o.counts, o.tables, o.headers, o.header_len, o.dht_off, o.dht_end);
 }
 
 static void launch_entropy(const EncodeBatchDev &e, bool long_blocks, cudaStream_t s) {
@@ -981,7 +1094,8 @@ enum class EncodeSource {
 // kernel stream only - for the bit totals that size the byte buffers, and for the file lengths - which the copies on
 // the other two streams do not notice.  Uploaded frames and finished files are double-buffered on the device.
 int encode_frames(hcj_ctx *c, EncodeSource kind, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
-                  int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len, int *status) {
+                  int restart_interval, bool optimize, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
+                  int *status) {
   CU_TRY(cudaSetDevice(c->device));
   int chunk = 64;
   if (const char *ev = getenv("HCJ_ENC_CHUNK")) chunk = std::max(1, atoi(ev));
@@ -1014,6 +1128,27 @@ int encode_frames(hcj_ctx *c, EncodeSource kind, const uint8_t *const *yuv, int 
   if (kind != EncodeSource::RGB_DEVICE) {
     if (nchunks > 1) alloc_owned((void **)&src_slot[1], slot_frame * (uint64_t)ch + 16);
     else src_slot[1] = src_slot[0];
+  }
+  // HCJ_ENC_OPTIMIZE_HUFFMAN: counts, tables and headers of one chunk (the kernel stream runs the chunks one after the
+  // other, so one set serves them all); the frames' headers are never longer than the shared one, which sizes out_stride
+  hcjk::HuffOpt opt = {};
+  if (optimize) {
+    const std::vector<uint8_t> &hd = S.header;
+    uint32_t p = 2;  // after SOI: segments up to the first DHT, then the DHT segments
+    while (p + 4 <= hd.size() && hd[p + 1] != 0xc4) p += 2 + ((hd[p + 2] << 8) | hd[p + 3]);
+    opt.dht_off = p;
+    while (p + 4 <= hd.size() && hd[p + 1] == 0xc4) p += 2 + ((hd[p + 2] << 8) | hd[p + 3]);
+    opt.dht_end = p;
+    e.tab_stride = 32 + 512;
+    e.frame_header_stride = hcj::align_up(e.header_len, 16);
+    alloc_owned((void **)&opt.counts, (uint64_t)ch * 4 * 256 * 4);
+    alloc_owned((void **)&opt.tables, (uint64_t)ch * e.tab_stride * 4);
+    alloc_owned((void **)&opt.headers, (uint64_t)ch * e.frame_header_stride);
+    alloc_owned((void **)&opt.header_len, 4 * (uint64_t)ch);
+    e.dc_codes = opt.tables;
+    e.ac_codes = opt.tables + 32;
+    e.frame_header = opt.headers;
+    e.frame_header_len = opt.header_len;
   }
   // k_rgb_to_ycc's frame table: the frames of both slots, or every caller frame (chunk k reads entries k * ch ..)
   const uint8_t **d_frames = nullptr;
@@ -1057,11 +1192,13 @@ int encode_frames(hcj_ctx *c, EncodeSource kind, const uint8_t *const *yuv, int 
     if (err == cudaSuccess) err = cudaStreamWaitEvent(s, ev_up[k], 0);
     if (err == cudaSuccess) err = cudaMemsetAsync(S.d_status, 0, 4 * (size_t)m, s);
     if (err == cudaSuccess) err = cudaMemsetAsync(e.long_blocks, 0, 4, s);
+    if (optimize && err == cudaSuccess) err = cudaMemsetAsync(opt.counts, 0, (size_t)m * 4 * 256 * 4, s);
     cudaEventRecord(ev_t[4 * k + 0], s);
     if (rgb)
       hcjk::launch_rgb_to_ycc(d_frames + (kind == EncodeSource::RGB_HOST ? (k & 1) * ch : lo), m, width, height, chroma,
                               const_cast<uint8_t *>(e.src), s);
     hcjk::launch_encode(e, s);
+    if (optimize) hcjk::launch_huff_opt(e, opt, S.d_status, s);
     hcjk::launch_bit_lengths(e, S.d_status, e.out_len, s);
     cudaEventRecord(ev_t[4 * k + 1], s);
     if (err == cudaSuccess) err = cudaGetLastError();
@@ -1137,15 +1274,24 @@ extern "C" {
 int hcj_encode_batch(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
                      int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len, int *status) {
   if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!yuv || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
-  return encode_frames(c, EncodeSource::YUV_HOST, yuv, n, width, height, chroma, quality, restart_interval, out, out_capacity,
+  return encode_frames(c, EncodeSource::YUV_HOST, yuv, n, width, height, chroma, quality, restart_interval, false, out, out_capacity,
                        out_len, status);
+}
+
+int hcj_encode_batch_ex(hcj_ctx *c, const uint8_t *const *yuv, int n, int width, int height, int chroma, int quality,
+                        int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
+                        int *status) {
+  if (flags & ~HCJ_ENC_OPTIMIZE_HUFFMAN) return HCJ_ERR_INVALID_ARG;
+  if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!yuv || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
+  return encode_frames(c, EncodeSource::YUV_HOST, yuv, n, width, height, chroma, quality, restart_interval,
+                       (flags & HCJ_ENC_OPTIMIZE_HUFFMAN) != 0, out, out_capacity, out_len, status);
 }
 
 int hcj_encode_rgb_batch(hcj_ctx *c, const uint8_t *const *rgb, int n, int width, int height, int chroma, int quality,
                          int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
                          int *status) {
   if (!c || n < 0 || n > HCJ_MAX_BATCH || (n > 0 && (!rgb || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
-  if (flags & ~HCJ_ENC_SRC_DEVICE) return HCJ_ERR_INVALID_ARG;
+  if (flags & ~(HCJ_ENC_SRC_DEVICE | HCJ_ENC_OPTIMIZE_HUFFMAN)) return HCJ_ERR_INVALID_ARG;
   if (flags & HCJ_ENC_SRC_DEVICE) {  // every frame must be device (or managed) memory of the context's device
     for (int i = 0; i < n; i++) {
       cudaPointerAttributes at;
@@ -1157,7 +1303,7 @@ int hcj_encode_rgb_batch(hcj_ctx *c, const uint8_t *const *rgb, int n, int width
     }
   }
   return encode_frames(c, (flags & HCJ_ENC_SRC_DEVICE) ? EncodeSource::RGB_DEVICE : EncodeSource::RGB_HOST, rgb, n, width, height,
-                       chroma, quality, restart_interval, out, out_capacity, out_len, status);
+                       chroma, quality, restart_interval, (flags & HCJ_ENC_OPTIMIZE_HUFFMAN) != 0, out, out_capacity, out_len, status);
 }
 
 int hcj_rgb_to_yuv(hcj_ctx *c, const uint8_t *rgb, int width, int height, int chroma, uint8_t *dst, size_t dst_capacity) {
@@ -1193,6 +1339,14 @@ int hcj_rgb_to_yuv(hcj_ctx *c, const uint8_t *rgb, int width, int height, int ch
 int hcj_encode_batch_multi(hcj_ctx *const *ctx, int nctx, const uint8_t *const *yuv, int n, int width, int height, int chroma,
                            int quality, int restart_interval, uint8_t *const *out, const size_t *out_capacity, size_t *out_len,
                            int *status) {
+  return hcj_encode_batch_multi_ex(ctx, nctx, yuv, n, width, height, chroma, quality, restart_interval, 0u, out, out_capacity,
+                                   out_len, status);
+}
+
+int hcj_encode_batch_multi_ex(hcj_ctx *const *ctx, int nctx, const uint8_t *const *yuv, int n, int width, int height, int chroma,
+                              int quality, int restart_interval, unsigned flags, uint8_t *const *out, const size_t *out_capacity,
+                              size_t *out_len, int *status) {
+  if (flags & ~HCJ_ENC_OPTIMIZE_HUFFMAN) return HCJ_ERR_INVALID_ARG;
   if (!ctx || nctx < 1 || n < 0 || (n > 0 && (!yuv || !out || !out_capacity || !out_len))) return HCJ_ERR_INVALID_ARG;
   for (int k = 0; k < nctx; k++) {
     if (!ctx[k]) return HCJ_ERR_INVALID_ARG;
@@ -1203,8 +1357,8 @@ int hcj_encode_batch_multi(hcj_ctx *const *ctx, int nctx, const uint8_t *const *
   auto work = [&](int k) {
     int lo, hi;
     hcj_shard_range(n, k, nctx, &lo, &hi);
-    rc[k] = hcj_encode_batch(ctx[k], yuv + lo, hi - lo, width, height, chroma, quality, restart_interval, out + lo, out_capacity + lo,
-                             out_len + lo, status ? status + lo : nullptr);
+    rc[k] = hcj_encode_batch_ex(ctx[k], yuv + lo, hi - lo, width, height, chroma, quality, restart_interval, flags, out + lo,
+                                out_capacity + lo, out_len + lo, status ? status + lo : nullptr);
   };
   std::vector<std::thread> pool;
   try {

@@ -153,6 +153,11 @@ struct EncodeBatchDev {
   uint32_t *long_blocks;      // != 0: some block of the chunk is longer than its slot (k_pack has work)
   const uint8_t *header;      // shared header bytes
   uint32_t header_len;
+  // HCJ_ENC_OPTIMIZE_HUFFMAN: per-frame tables and headers (k_huff_tables)
+  uint32_t tab_stride;            // frame f codes with dc_codes / ac_codes + f * tab_stride (0: the shared default tables)
+  const uint8_t *frame_header;    // [n][frame_header_stride] header of every frame, or null: the shared header
+  uint64_t frame_header_stride;
+  const uint32_t *frame_header_len;  // [n]
 };
 void launch_encode(const EncodeBatchDev &e, cudaStream_t s);
 void launch_encode_block_log(const EncodeBatchDev &e, uint32_t first, uint32_t count, void *out /* hcj_encoder_block[count] */, cudaStream_t s);

@@ -32,6 +32,7 @@ FLAG_SCALE_MASK = 0x30
 # RGB24 equals Pillow / OpenCV.  Not combinable with FLAG_SCALE_*.
 FLAG_LIBJPEG = 0x40
 ENC_SRC_DEVICE = 1  # hcj_encode_rgb_batch: the frames are device pointers on the context's device
+ENC_OPTIMIZE_HUFFMAN = 0x100  # every frame with its own optimal Huffman tables (include/hcjpeg.h)
 
 MAX_COMPONENTS = 4
 MAX_TABLE_SEGMENTS = 64
@@ -182,6 +183,8 @@ _SIGS = {
     "hcj_batch_fetch_coefficients": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]),
     "hcj_batch_fetch_entropy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, _P(C.c_size_t)]),
     "hcj_idct_blocks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "hcj_encode_batch_ex": (C.c_int, [C.c_void_p, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
+    "hcj_encode_batch_multi_ex": (C.c_int, [_P(C.c_void_p), C.c_int, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
     "hcj_encode_batch": (C.c_int, [C.c_void_p, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
     "hcj_encode_rgb_batch": (C.c_int, [C.c_void_p, _P(C.c_void_p), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, _P(C.c_void_p), _P(C.c_size_t), _P(C.c_size_t), _P(C.c_int)]),
     "hcj_rgb_to_yuv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t]),
@@ -469,21 +472,22 @@ class Context:
         return out
 
     # ---- encode -----------------------------------------------------------------------------
-    def encode_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None):
-        """Encoder.encode_420/422/444 for every raw planar frame (bytes / uint8 arrays) in ``frames``."""
-        return self._encode(frames, None, width, height, chroma, quality, restart_interval, capacity)
+    def encode_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None, optimize=False):
+        """Encoder.encode_420/422/444 for every raw planar frame (bytes / uint8 arrays) in ``frames`` (hcj_encode_batch_ex).
+        optimize=True: every frame with its own optimal Huffman tables (ENC_OPTIMIZE_HUFFMAN)."""
+        return self._encode(frames, None, width, height, chroma, quality, restart_interval, capacity, optimize)
 
-    def encode_rgb_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None):
+    def encode_rgb_batch(self, frames, width, height, chroma=420, quality=75, restart_interval=0, capacity=None, optimize=False):
         """hcj_encode_rgb_batch: every RGB24 frame converted and sub-sampled to ``chroma`` on the device (the stated forward
         formula, include/hcjpeg.h) and encoded as encode_batch encodes that planar frame.  ``frames``: all host frames
         (bytes of width*height*3, or C-contiguous uint8 arrays of shape (height, width, 3)) or all device frames (objects
         with ``__cuda_array_interface__`` of that shape, e.g. torch CUDA tensors, read on the context's stream).
-        Returns (files, status) like encode_batch."""
+        Returns (files, status) like encode_batch; optimize=True as there."""
         ptrs, flags = _rgb_frames(frames, width, height)
-        return self._encode(ptrs, flags, width, height, chroma, quality, restart_interval, capacity)
+        return self._encode(ptrs, flags, width, height, chroma, quality, restart_interval, capacity, optimize)
 
-    def _encode(self, frames, rgb_flags, width, height, chroma, quality, restart_interval, capacity):
-        """hcj_encode_batch (rgb_flags None) or hcj_encode_rgb_batch with those flags."""
+    def _encode(self, frames, rgb_flags, width, height, chroma, quality, restart_interval, capacity, optimize=False):
+        """hcj_encode_batch_ex (rgb_flags None) or hcj_encode_rgb_batch with those flags."""
         n = len(frames)
         auto = capacity is None
         if auto:
@@ -494,15 +498,17 @@ class Context:
         caps = (C.c_size_t * max(n, 1))(*([capacity] * n))
         lens = (C.c_size_t * max(n, 1))()
         status = (C.c_int * max(n, 1))()
+        opt = ENC_OPTIMIZE_HUFFMAN if optimize else 0
         if rgb_flags is None:
             _check(
-                lib().hcj_encode_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, op, caps, lens, status),
-                "hcj_encode_batch",
+                lib().hcj_encode_batch_ex(self._h, fp, n, width, height, chroma, quality, restart_interval, opt, op, caps, lens,
+                                          status),
+                "hcj_encode_batch_ex",
             )
         else:
             _check(
-                lib().hcj_encode_rgb_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, rgb_flags, op, caps,
-                                           lens, status),
+                lib().hcj_encode_rgb_batch(self._h, fp, n, width, height, chroma, quality, restart_interval, rgb_flags | opt, op,
+                                           caps, lens, status),
                 "hcj_encode_rgb_batch",
             )
         st = [status[i] for i in range(n)]
@@ -512,7 +518,8 @@ class Context:
         redo = [i for i in range(n) if st[i] == -30] if auto else []
         if redo:
             again, st2 = self._encode(
-                [frames[i] for i in redo], rgb_flags, width, height, chroma, quality, restart_interval, max(lens[i] for i in redo)
+                [frames[i] for i in redo], rgb_flags, width, height, chroma, quality, restart_interval, max(lens[i] for i in redo),
+                optimize,
             )
             for i, o, s2 in zip(redo, again, st2):
                 res[i], st[i] = o, s2
@@ -613,8 +620,8 @@ def decode_batch_multi(ctxs, jpegs, mode=OUT_YUV, flags=FLAG_DEFAULT):
     return [outs[i][: caps[i]] if st[i] == 0 else None for i in range(n)], st
 
 
-def encode_batch_multi(ctxs, frames, width, height, chroma=420, quality=75, restart_interval=0):
-    """hcj_encode_batch_multi: frames sharded by index over one Context per GPU."""
+def encode_batch_multi(ctxs, frames, width, height, chroma=420, quality=75, restart_interval=0, optimize=False):
+    """hcj_encode_batch_multi_ex: frames sharded by index over one Context per GPU; optimize=True as in encode_batch."""
     n = len(frames)
     capacity = lib().hcj_encode_bound(width, height, chroma) if n <= 64 else width * height * 3 + (1 << 16)
     outs = [np.zeros(capacity, np.uint8) for _ in range(n)]
@@ -624,8 +631,9 @@ def encode_batch_multi(ctxs, frames, width, height, chroma=420, quality=75, rest
     lens = (C.c_size_t * max(n, 1))()
     status = (C.c_int * max(n, 1))()
     hs = (C.c_void_p * len(ctxs))(*[c._h.value for c in ctxs])
-    _check(lib().hcj_encode_batch_multi(hs, len(ctxs), fp, n, width, height, chroma, quality, restart_interval, op, caps, lens, status),
-           "hcj_encode_batch_multi")
+    _check(lib().hcj_encode_batch_multi_ex(hs, len(ctxs), fp, n, width, height, chroma, quality, restart_interval,
+                                           ENC_OPTIMIZE_HUFFMAN if optimize else 0, op, caps, lens, status),
+           "hcj_encode_batch_multi_ex")
     st = [status[i] for i in range(n)]
     return [outs[i][: lens[i]].tobytes() if st[i] == 0 else None for i in range(n)], st
 
